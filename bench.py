@@ -3,10 +3,12 @@
 HBM GB/s vs peak) on N GPUs of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c2|c1|c3|c4|c5] [--batch B] [--no-sweep] ...
+                    [--workload c2|c1|c3|c4|c5] [--batch B] [--no-sweep] [--dump-outputs DIR] ...
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
-A "step" is one pass of the hot path over one batch of synthetic input.  Workloads = BASELINE.json configs:
+A "step" is one pass of the hot path over one batch of synthetic input; the timed region is exactly --steps steps.
+`--dump-outputs DIR` writes what the last timed step computed (c4: the frames and label maps of the rollout; otherwise
+the loss vector and the gradients to flow, src_rgb and src_layout) as DIR/<name>.npy.  Workloads = BASELINE.json configs:
   c2 (default)  16x256x512, K=20, fp32: flow-guided warp of RGB + layout, all loss terms, gradients to flow, src_rgb and
                 src_layout (220 algorithmic B/px).  Weak scaling: every rank processes one such batch; the only exchange
                 is one NCCL all-reduce of the 8-float loss vector.
@@ -37,6 +39,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOADS = {
@@ -57,8 +60,10 @@ BYTES_PER_PX = {"f32": dict(step=220, pass1=128, rgb_strip=32, lay_tile=96, pass
                 "bf16": dict(step=122, pass1=76, rgb_strip=20, lay_tile=56, pass2=46)}
 ROLLOUT_BYTES_PER_PX = 48      # per rollout step: coords 8 + rgb 12 + label 8 read, rgb 12 + label 8 written
 FALLBACK_HBM_GBS = 6650.0
-MIN_TIMED_MS = 250.0           # the timed region lasts at least this long whatever --steps says
+WARM_MS = 250.0                # untimed passes right before every timed region
 REF_SAMPLE_IMAGES = 2          # bounded sample of the CPU arms (cpu_baseline and --impl reference alike)
+DUMP_LIMIT_BYTES = 64 * 10**6  # --dump-outputs: all files together
+DUMP_SEED = 1024
 
 
 def make_inputs(N, H, W, K, sigma, far, dtype, device, seed=1024):
@@ -254,9 +259,11 @@ class Ctx:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return t.item()
 
-    def timed(self, step, steps, min_ms=MIN_TIMED_MS):
-        """EXACTLY `steps` step groups of `r` passes each between barrier + synchronize on both sides; `r` is chosen
-        so that the region lasts >= min_ms.  Returns (ms per pass, max over ranks; r; ms of the whole region)."""
+    def timed(self, step, steps, min_ms=0.0):
+        """EXACTLY `steps` step groups of `r` passes each, ending in a barrier + synchronize; `r` is 1 unless `min_ms` > 0,
+        then it is chosen so that the region lasts >= min_ms.  Right before the region, WARM_MS of passes bring the clocks
+        back up after whatever idle gap preceded the call, so that a short region is not timed at idle clocks.  Returns
+        (ms per pass, max over ranks; r; ms of the whole region)."""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         self.barrier()
         e0.record(self.stream)
@@ -264,10 +271,15 @@ class Ctx:
             step(i)
         e1.record(self.stream)
         self.barrier()
-        est_ms = self.max_over_ranks(e0.elapsed_time(e1) / 4)
-        r = max(1, int(math.ceil(min_ms / max(est_ms * steps, 1e-6))))
+        est_ms = max(self.max_over_ranks(e0.elapsed_time(e1) / 4), 1e-6)
+        r = max(1, int(math.ceil(min_ms / (est_ms * steps))))
+        for i in range(int(math.ceil(WARM_MS / est_ms))):
+            step(i)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        self.barrier()
+        # ranks start the region together; a single process leaves the warm-up queued ahead of e0 instead, so that the
+        # GPU does not idle for a launch between e0 and the first timed pass (a visible share of a region of a few steps)
+        if self.dist is not None:
+            self.barrier()
         e0.record(self.stream)
         for i in range(steps * r):
             step(i)
@@ -566,7 +578,9 @@ class Rollout:
         del d
 
     def step(self, i=0):
-        return self.cx.vlg.rollout(self.img, self.lab, lambda t, im, lb: self.flows[t], steps=ROLLOUT_STEPS)
+        """One rollout; its (frames, label maps) stay in `self.out` until the next one."""
+        self.out = self.cx.vlg.rollout(self.img, self.lab, lambda t, im, lb: self.flows[t], steps=ROLLOUT_STEPS)
+        return self.out
 
     def e2e(self, steps):
         """Uploads the uint8 start frame + class map and the five fp32 flows, rolls out, reads the final class map back
@@ -680,6 +694,22 @@ def sweep_variants_c2(cx, peak):
     return out
 
 
+def dump_outputs(outdir, arrays):
+    """Writes every tensor of `arrays` as outdir/<name>.npy in float32.  Each array gets an equal share of
+    DUMP_LIMIT_BYTES; a larger one is written as a fixed, seeded sample of its elements (sorted flat indices into its
+    logical shape, e.g. NCHW whatever the memory format), so two runs with the same arguments compare element for
+    element."""
+    os.makedirs(outdir, exist_ok=True)
+    share = (DUMP_LIMIT_BYTES // len(arrays) - 128) // 4      # elements per array; 128 bytes of .npy header
+    g = torch.Generator().manual_seed(DUMP_SEED)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > share:
+            idx = torch.randint(0, t.numel(), (share,), generator=g).sort().values.to(t.device)
+            t = t[torch.unravel_index(idx, t.shape)]
+        np.save(os.path.join(outdir, name + ".npy"), t.float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -695,6 +725,8 @@ def main():
     ap.add_argument("--no-sweep", action="store_true", help="skip the compact lines of the other BASELINE configs")
     ap.add_argument("--no-aux", action="store_true", help="skip the boundary-fusion / forward-warp side measurements")
     ap.add_argument("--flow-grad-only", action="store_true", help="sources are data: no d_src (128 B/px variant)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32, "
+                    "<= 64 MB in all; larger outputs as a fixed, seeded sample)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -727,6 +759,10 @@ def main():
             sampler.start(); sampler.wait_first()
         ms, r, total = cx.timed(ro.step, args.steps)
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:
+            imgs, labs = ro.out
+            dump_outputs(args.dump_outputs, {**{f"frame{t + 1}": x for t, x in enumerate(imgs)},
+                                             **{f"label{t + 1}": x for t, x in enumerate(labs)}})
         e2e = ro.e2e(args.steps)
         if rank != 0:
             if dist is not None: dist.destroy_process_group()
@@ -764,6 +800,9 @@ def main():
         sampler.start(); sampler.wait_first()
     ms_per_step, replays, timed_ms = cx.timed(fz.step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # the buffers of the last timed step, before anything launches again
+        outs = {"loss": fz.loss, "d_flow": fz.d_c, "d_src_rgb": fz.d_a, "d_src_layout": fz.d_b}
+        dump_outputs(args.dump_outputs, {k: v for k, v in outs.items() if v is not None})
     launches = fz.count_launches(args.steps * replays)
 
     # ---- per-kernel device times inside the direct launch sequence (CUDA events on the launch stream) ----
@@ -895,8 +934,7 @@ def main():
                    "l2_policy": "inputs (%.0f MB/step) exceed the 126 MB L2; two input sets alternate" % (P * 120 / 1e6),
                    "launch": "cuda graph replay" if graph_used else "direct launches",
                    "replays_per_step": replays, "timed_region_ms": timed_ms,
-                   "timing_note": f"the timed region is {args.steps} step groups of {replays} passes each (>= {MIN_TIMED_MS:.0f} ms); "
-                                  "ms_per_step is per single pass",
+                   "timing_note": f"the timed region is {args.steps} steps; ms_per_step is per step",
                    "exchange": ("one NCCL all-reduce of the 8-float loss vector per step, issued after pass 1 and overlapped with pass 2"
                                 if world > 1 else "none (single GPU)")},
         "roofline": {"bound": "hbm", "kernel": dom, "achieved": achieved, "peak": peak, "unit": "GB/s",
