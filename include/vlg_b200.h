@@ -110,7 +110,8 @@ typedef struct vlg_problem {
     uint32_t flags;       /* VLG_FLAG_*                                                            */
     int64_t ignore_index; /* nn.CrossEntropyLoss default -100 (src/trainer.py:124)                 */
     float w_l1, w_gd, w_ssim, w_ce, w_tv; /* 40, 20, 20, 10 (src/trainer.py:248-250) + TV weight  */
-    uint32_t term_mask;   /* VLG_TERM_* bits to evaluate; 0 = all.  Skipped terms read as 0.       */
+    uint32_t term_mask;   /* VLG_TERM_* bits to evaluate; 0 = all.  Skipped terms read as 0 and add
+                           * nothing to the total or to any gradient, whatever their weight.        */
     uint32_t ce_norm;     /* VLG_CE_NORM_*: divisor of the (weighted) cross-entropy sum                 */
     /* Divisors of the means.  0 = derive from N,H,W (single GPU).  Data-parallel ranks pass the
      * GLOBAL batch here so that per-rank loss vectors and gradients simply add (SURVEY 8e). */

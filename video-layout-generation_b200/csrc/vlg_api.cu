@@ -249,6 +249,7 @@ static ReduceParams make_reduce_params(const vlg_problem_t *prob, const WsLayout
     rp.ce_scale = (double)prob->N / Ng;
     rp.w_l1 = prob->w_l1; rp.w_gd = prob->w_gd; rp.w_ssim = prob->w_ssim; rp.w_ce = prob->w_ce; rp.w_tv = prob->w_tv;
     rp.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
+    rp.ce_on = !prob->term_mask || (prob->term_mask & VLG_TERM_CE);
     rp.out = loss_out;   // NULL: pass 1 does not fuse the final reduction
     return rp;
 }
@@ -786,7 +787,8 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     pp.do_tv = warp && prob->coord_mode == VLG_COORD_FLOW && (pp.terms & VLG_TERM_TV);
     pp.c_tvh = prob->H > 1 ? (float)(prob->w_tv / (Ng * (H - 1) * W * 2)) : 0.f;
     pp.c_tvw = prob->W > 1 ? (float)(prob->w_tv / (Ng * H * (W - 1) * 2)) : 0.f;
-    pp.w_ce_over_scale = (float)(prob->w_ce * (double)prob->N / Ng);
+    // a masked-out CE still runs its forward sum (the reduction drops it) but sends no gradient anywhere
+    pp.w_ce_over_scale = (pp.terms & VLG_TERM_CE) ? (float)(prob->w_ce * (double)prob->N / Ng) : 0.f;
     pp.need_grad = need_grad;
     pp.d_coords = d_coords; pp.d_out_rgb = d_out_rgb; pp.d_out_lay = d_out_lay;
     pp.out_argmax = out_argmax;
@@ -935,7 +937,7 @@ static int run_pass1_labels(const vlg_problem_t *prob, const void *src_rgb, cons
     lp.src_label = src_label; lp.coords = (const float2 *)coords; lp.tgt_label = tgt_label; lp.ignore_index = prob->ignore_index;
     lp.class_weight = prob->ce_class_weight;
     lp.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
-    lp.w_ce_over_scale = (float)(prob->w_ce * (double)prob->N / Ng);
+    lp.w_ce_over_scale = (terms & VLG_TERM_CE) ? (float)(prob->w_ce * (double)prob->N / Ng) : 0.f;   // see run_pass1
     lp.do_tv = prob->coord_mode == VLG_COORD_FLOW && (terms & VLG_TERM_TV);
     lp.c_tvh = prob->H > 1 ? (float)(prob->w_tv / (Ng * (H - 1) * W * 2)) : 0.f;
     lp.c_tvw = prob->W > 1 ? (float)(prob->w_tv / (Ng * H * (W - 1) * 2)) : 0.f;

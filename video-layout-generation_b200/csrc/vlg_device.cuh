@@ -53,6 +53,7 @@ struct ReduceParams {
     double ce_scale;        // N_local/N_global
     float w_l1, w_gd, w_ssim, w_ce, w_tv;
     int weighted_denom;     // 1: CE divisor = hdr->ce_denom (class-weighted torch mean), 0: n_valid
+    int ce_on;              // VLG_TERM_CE is evaluated; 0: the CE slot reads 0 and stays out of the total
     float *out;
 };
 
@@ -88,7 +89,7 @@ __device__ __forceinline__ void reduce_partials_block(const ReduceParams &p, dou
         const double l1 = s[0] * p.inv_numel_rgb, gd = s[NT] * p.inv_numel_rgb;
         const double ssim = s[2 * NT] * p.inv_ssim;
         const double cd = p.weighted_denom ? __ldcg(&p.hdr->ce_denom) : nv;
-        const double ce = cd > 0 ? s[3 * NT] / cd * p.ce_scale : 0.0;
+        const double ce = (p.ce_on && cd > 0) ? s[3 * NT] / cd * p.ce_scale : 0.0;
         const double tv = s[4 * NT] * p.inv_tvh + s[5 * NT] * p.inv_tvw;
         p.out[VLG_LOSS_L1] = (float)l1;
         p.out[VLG_LOSS_GD] = (float)gd;
