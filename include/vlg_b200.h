@@ -54,8 +54,6 @@ extern "C" {
 /* flags */
 #define VLG_FLAG_NO_FAR_PATH 1u /* caller asserts |displacement| < VLG_NEAR_RADIUS; far taps raise status */
 #define VLG_FLAG_NO_TMA 2u      /* stage the source-layout window with cp.async instead of a TMA tensor map   */
-#define VLG_FLAG_TILE_RGB 4u    /* evaluate the rgb terms in the tile kernel instead of the column-strip kernel */
-#define VLG_FLAG_TILE_LAYOUT 8u /* evaluate the layout terms in the first (non-persistent) tile kernel            */
 #define VLG_FLAG_FAR_WIDE 64u     /* far path: always one 64-bit accumulator per channel (default: two 32-bit lanes per 64-bit word in
                                    * every source-tile row that receives at most 512 far pixels)                                 */
 #define VLG_FLAG_PASS2_COORDS 32u /* pass 2 re-derives the tap cells and weights from the coordinates and scans (pass2_kernel)

@@ -69,7 +69,6 @@ def test_python_constants_match_the_header():
     """Every VLG_FLAG_* / VLG_TERM_* / VLG_STATUS_* / VLG_CE_NORM_* / VLG_NEAR_RADIUS the Python side mirrors has the
     value the header (as gcc sees it) gives it -- a flag added on one side only would silently select another path."""
     names = {"VLG_FLAG_NO_FAR_PATH": _cabi.FLAG_NO_FAR_PATH, "VLG_FLAG_NO_TMA": _cabi.FLAG_NO_TMA,
-             "VLG_FLAG_TILE_RGB": _cabi.FLAG_TILE_RGB, "VLG_FLAG_TILE_LAYOUT": _cabi.FLAG_TILE_LAYOUT,
              "VLG_FLAG_PASS2_COORDS": _cabi.FLAG_PASS2_COORDS, "VLG_FLAG_FAR_WIDE": _cabi.FLAG_FAR_WIDE,
              "VLG_TERM_L1": _cabi.TERM_L1, "VLG_TERM_GD": _cabi.TERM_GD, "VLG_TERM_SSIM": _cabi.TERM_SSIM,
              "VLG_TERM_CE": _cabi.TERM_CE, "VLG_TERM_TV": _cabi.TERM_TV,
@@ -146,6 +145,12 @@ def test_argument_validation_without_gpu():
     assert big >= P * 23 * 4 + P * 23 * 8
     ok.flags = _cabi.FLAG_NO_FAR_PATH
     assert lib.vlg_workspace_bytes(C.byref(ok), 1) < big
+    # bits 4 and 8 selected pass-1 organisations that are retired; unknown bits are refused, not ignored
+    for retired in (4, 8, 4 | 8, 128):
+        unknown = _cabi.Problem(N=2, H=128, W=256, K=20, padding=1, flags=_cabi.FLAG_NO_TMA | retired)
+        assert lib.vlg_workspace_bytes(C.byref(unknown), 0) == 0
+        assert b"unknown flag bits" in lib.vlg_last_error()
+        assert b"VLG_FLAG_TILE_RGB" in lib.vlg_last_error() and b"VLG_FLAG_TILE_LAYOUT" in lib.vlg_last_error()
     # NULL workspace is refused before anything is launched
     rc = lib.vlg_reduce_partials(C.byref(ok), None, None, 0, None)
     assert rc == -1

@@ -43,10 +43,8 @@ REACH = {"l1": (True, True, False), "gd": (True, True, False), "ssim": (True, Tr
          "ce": (True, False, True), "tv": (True, False, False)}
 
 ORGS = {
-    "default": {},                               # rgb_strip_kernel + lay_tile_kernel (K % 4 == 0)
-    "tile": dict(layout_kernel="tile"),          # rgb_strip_kernel + pass1_kernel for the layout
-    "tile_kernels": dict(tile_kernels=True),     # everything in pass1_kernel
-    "no_tma": dict(use_tma=False),               # cp.async staging of the layout window
+    "default": {},                               # rgb_strip_kernel + lay_tile_kernel (K % 4 == 0), else + pass1_kernel
+    "no_tma": dict(use_tma=False),               # rgb_strip_kernel + pass1_kernel (cp.async staging of the layout window)
     "no_records": dict(pass2_records=False),     # pass 2 re-derives its taps from the coordinates
 }
 
@@ -137,10 +135,10 @@ FUSED = [
     ("default", 19, "squeeze", "zeros", (1, 9, 33)),
     ("default", 20, "far", "zeros", (2, 67, 129)),
     ("default", 20, "far_wide", "border", (3, 24, 84)),
-    ("tile", 20, "squeeze", "zeros", (3, 24, 84)),
-    ("tile", 19, "far", "border", (2, 17, 57)),
-    ("tile_kernels", 20, "far", "border", (2, 67, 129)),
-    ("tile_kernels", 19, "near", "zeros", (1, 9, 33)),
+    ("no_tma", 20, "squeeze", "zeros", (3, 24, 84)),
+    ("default", 19, "far", "border", (2, 17, 57)),
+    ("no_tma", 20, "far", "border", (2, 67, 129)),
+    ("default", 30, "near", "zeros", (1, 9, 33)),
     ("no_tma", 20, "near", "zeros", (2, 67, 129)),
     ("no_tma", 19, "far_wide", "border", (3, 24, 84)),
     ("no_records", 20, "far_wide", "zeros", (1, 9, 33)),

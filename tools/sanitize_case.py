@@ -31,11 +31,12 @@ for (N, H, W, sigma, far) in ((1, 37, 70, 1.5, 0.0), (2, 24, 45, 6.0, 0.05)):
     fr = torch.rand(N, 3, H, W, device=dev)
     vlg_b200.prepare_frames(fr, flip=True, labels=lab)
     vlg_b200.prepare_frames(cl(fr.cpu()), denormalize=True, dtype=torch.bfloat16)
-    # bf16 layouts (8-byte-unit TMA map), pass 2 from coordinates, other pass-1 organisations
+    # bf16 layouts (8-byte-unit TMA map when W is even; pass1_kernel + tap_records_kernel for W = 45), pass 2 from
+    # coordinates, the layout terms in pass1_kernel (cp.async staging)
     a16, b16 = a.detach().to(torch.bfloat16).requires_grad_(True), b.detach().to(torch.bfloat16).requires_grad_(True)
     total, _, _ = vlg_b200.warp_loss(a16, b16, f, t.to(torch.bfloat16), lab, vlg_b200.WarpLossConfig(w_tv=0.5))
     total.backward()
-    for kw in (dict(pass2_records=False), dict(layout_kernel="tile"), dict(tile_kernels=True)):
+    for kw in (dict(pass2_records=False), dict(use_tma=False)):
         total, _, _ = vlg_b200.warp_loss(a, b, f, t, lab, vlg_b200.WarpLossConfig(w_tv=0.5, **kw))
         total.backward()
     # label-source op and uint8 ingest

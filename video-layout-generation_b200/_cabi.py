@@ -11,8 +11,6 @@ PAD_ZEROS, PAD_BORDER = 0, 1
 COORD_FLOW, COORD_GRID = 0, 1
 FLAG_NO_FAR_PATH = 1
 FLAG_NO_TMA = 2
-FLAG_TILE_RGB = 4
-FLAG_TILE_LAYOUT = 8
 FLAG_PASS2_COORDS = 32
 FLAG_FAR_WIDE = 64
 TERM_L1, TERM_GD, TERM_SSIM, TERM_CE, TERM_TV, TERM_ALL = 1, 2, 4, 8, 16, 31

@@ -129,6 +129,10 @@ static int check_problem(const vlg_problem_t *p) {
     if (p->global_N != 0 && p->global_N < p->N) return fail(VLG_ERR_ARG, "global_N < N");
     if (p->ce_norm != VLG_CE_NORM_TORCH && p->ce_norm != VLG_CE_NORM_COUNT) return fail(VLG_ERR_ARG, "bad ce_norm %u", p->ce_norm);
     if (p->ce_class_weight && p->K > 32) return fail(VLG_ERR_UNSUPPORTED, "class weights need K <= 32");
+    constexpr uint32_t known_flags = VLG_FLAG_NO_FAR_PATH | VLG_FLAG_NO_TMA | VLG_FLAG_PASS2_COORDS | VLG_FLAG_FAR_WIDE;
+    if (p->flags & ~known_flags)
+        return fail(VLG_ERR_ARG, "unknown flag bits 0x%x (4 and 8 were VLG_FLAG_TILE_RGB and VLG_FLAG_TILE_LAYOUT, which are retired)",
+                    p->flags & ~known_flags);
     return VLG_OK;
 }
 
@@ -234,7 +238,26 @@ __global__ void __launch_bounds__(256) reduce_partials_kernel(const ReduceParams
     reduce_partials_block<256>(p, s);
 }
 
-static ReduceParams make_reduce_params(const vlg_problem_t *prob, const WsLayout &L, char *ws, float *loss_out) {
+// The loss terms in effect and their coefficients.  `warp`: a warped step (TV is a term of the pixel flow only).
+static TermCoeffs make_terms(const vlg_problem_t *prob, bool warp) {
+    const double Ng = (double)(prob->global_N ? prob->global_N : prob->N);
+    const double H = (double)prob->H, W = (double)prob->W;
+    TermCoeffs tc{};
+    tc.terms = prob->term_mask ? prob->term_mask : VLG_TERM_ALL;
+    if (!(prob->H > 2 && prob->W > 2)) tc.terms &= ~VLG_TERM_SSIM;
+    if (!(warp && prob->coord_mode == VLG_COORD_FLOW)) tc.terms &= ~VLG_TERM_TV;
+    tc.c_l1 = (tc.terms & VLG_TERM_L1) ? (float)(prob->w_l1 / (Ng * 3 * H * W)) : 0.f;
+    tc.c_gd = (tc.terms & VLG_TERM_GD) ? (float)(prob->w_gd / (Ng * 3 * H * W)) : 0.f;
+    tc.c_ssim = (tc.terms & VLG_TERM_SSIM) ? (float)(prob->w_ssim / (2.0 * Ng * (H - 2) * (W - 2))) : 0.f;
+    tc.c_tvh = (tc.terms & VLG_TERM_TV) ? (float)(prob->w_tv / (Ng * (H - 1) * W * 2)) : 0.f;
+    tc.c_tvw = (tc.terms & VLG_TERM_TV) ? (float)(prob->w_tv / (Ng * H * (W - 1) * 2)) : 0.f;
+    // a masked-out CE still runs its forward sum (the reduction drops it) but sends no gradient anywhere
+    tc.w_ce_over_scale = (tc.terms & VLG_TERM_CE) ? (float)(prob->w_ce * (double)prob->N / Ng) : 0.f;
+    tc.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
+    return tc;
+}
+
+static ReduceParams make_reduce_params(const vlg_problem_t *prob, const TermCoeffs &tc, const WsLayout &L, char *ws, float *loss_out) {
     const double Ng = (double)(prob->global_N ? prob->global_N : prob->N);
     const double H = (double)prob->H, W = (double)prob->W;
     ReduceParams rp{};
@@ -248,8 +271,8 @@ static ReduceParams make_reduce_params(const vlg_problem_t *prob, const WsLayout
     rp.inv_tvw = 1.0 / (Ng * H * (W - 1) * 2);
     rp.ce_scale = (double)prob->N / Ng;
     rp.w_l1 = prob->w_l1; rp.w_gd = prob->w_gd; rp.w_ssim = prob->w_ssim; rp.w_ce = prob->w_ce; rp.w_tv = prob->w_tv;
-    rp.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
-    rp.ce_on = !prob->term_mask || (prob->term_mask & VLG_TERM_CE);
+    rp.weighted_denom = tc.weighted_denom;
+    rp.terms = tc.terms;
     rp.out = loss_out;   // NULL: pass 1 does not fuse the final reduction
     return rp;
 }
@@ -488,10 +511,10 @@ static EncodeTiledFn tensor_map_encoder() {
     return fn;
 }
 
-// Tensor map of the NHWC source layout [N][H][W][K] with a kSW x kSH x K box: the window a pass-1 CTA
-// stages.  Returns false when TMA cannot be used (bf16 K=20 rows are not 16-byte multiples, odd K, ...).
-static bool make_layout_map(const vlg_problem_t *prob, const void *src_layout, CUtensorMap *map, int box_w = kSW,
-                            int box_h = kSH, bool fp32_storage = false) {
+// Tensor map of an NHWC layout [N][H][W][K] with a box_w x box_h x K box.  Returns false when TMA cannot be used
+// (bf16 K=20 rows are not 16-byte multiples, odd K, ...).
+static bool make_layout_map(const vlg_problem_t *prob, const void *src_layout, CUtensorMap *map, int box_w, int box_h,
+                            bool fp32_storage = false) {
     memset(map, 0, sizeof(*map));
     const size_t es = 4;
     if ((prob->dtype != VLG_F32 && !fp32_storage) || (prob->K * es) % 16 != 0 || prob->K > 256) return false;
@@ -557,7 +580,7 @@ static bool make_pitched_map(const vlg_problem_t *prob, const void *base, int64_
 }
 
 template <typename T, int K>
-static int launch_pass1(bool warp, const Pass1Params &pp, const CUtensorMap &lay_map, int64_t n_blocks, cudaStream_t st) {
+static int launch_pass1(bool warp, const Pass1Params &pp, cudaStream_t st) {
     // the staged source window is the last member: the un-warped criteria do not allocate it
     using Smem = Pass1Smem<T, K>;
     const size_t smem_warp = sizeof(Smem), smem_plain = offsetof(Smem, stage);
@@ -565,18 +588,15 @@ static int launch_pass1(bool warp, const Pass1Params &pp, const CUtensorMap &lay
     if (int rc = ensure_smem(attr_warp, pass1_kernel<T, K, true>, smem_warp, "pass1")) return rc;
     if (int rc = ensure_smem(attr_plain, pass1_kernel<T, K, false>, smem_plain, "pass1")) return rc;
     const dim3 grid((unsigned)pp.tiles_x, (unsigned)pp.tiles_y, (unsigned)pp.N);
-    (void)n_blocks;
-    if (warp) pass1_kernel<T, K, true><<<grid, kThreads, smem_warp, st>>>(pp, lay_map);
-    else pass1_kernel<T, K, false><<<grid, kThreads, smem_plain, st>>>(pp, lay_map);
+    if (warp) pass1_kernel<T, K, true><<<grid, kThreads, smem_warp, st>>>(pp);
+    else pass1_kernel<T, K, false><<<grid, kThreads, smem_plain, st>>>(pp);
     return check_launch("pass1_kernel");
 }
 
-static int dispatch_pass1(const vlg_problem_t *prob, bool warp, const Pass1Params &pp, const CUtensorMap &lay_map,
-                          int64_t n_blocks, cudaStream_t st) {
-#define X(k)                                                                              \
-    if (prob->K == k) {                                                                   \
-        return prob->dtype == VLG_F32 ? launch_pass1<float, k>(warp, pp, lay_map, n_blocks, st)    \
-                                      : launch_pass1<__nv_bfloat16, k>(warp, pp, lay_map, n_blocks, st); \
+static int dispatch_pass1(const vlg_problem_t *prob, bool warp, const Pass1Params &pp, cudaStream_t st) {
+#define X(k)                                                                                                              \
+    if (prob->K == k) {                                                                                                   \
+        return prob->dtype == VLG_F32 ? launch_pass1<float, k>(warp, pp, st) : launch_pass1<__nv_bfloat16, k>(warp, pp, st); \
     }
     VLG_FOR_EACH_K(X)
 #undef X
@@ -584,8 +604,7 @@ static int dispatch_pass1(const vlg_problem_t *prob, bool warp, const Pass1Param
 }
 
 template <typename T, int K>
-static int launch_pass2(Pass2Params pp, int64_t n_blocks, int64_t P, const vlg_problem_t *prob, size_t far_words, cudaStream_t st) {
-    (void)P; (void)far_words; (void)prob;
+static int launch_pass2(Pass2Params pp, const vlg_problem_t *prob, cudaStream_t st) {
     if (pp.far_acc) {   // both exit at once unless pass 1 queued far pixels
         const int sms = sm_count();
         far_zero_kernel<K><<<sms * 2, kThreads, 0, st>>>(pp);
@@ -615,7 +634,6 @@ static int launch_pass2(Pass2Params pp, int64_t n_blocks, int64_t P, const vlg_p
     constexpr size_t smem = pass2_smem_bytes<K>();
     static PerDevice attr;  // per instantiation
     if (int rc = ensure_smem(attr, pass2_kernel<T, K>, smem, "pass2")) return rc;
-    (void)n_blocks;
     // the fp32 d_out staging buffer as a [N][H][W][K] tensor with a kQW x kQH window box
     CUtensorMap dout_map;
     pp.use_tma = (pp.d_src_lay && pp.d_out_lay && !(prob->flags & VLG_FLAG_NO_TMA) &&
@@ -713,30 +731,84 @@ static int dispatch_laytile(const vlg_problem_t *prob, const LayParams &lp, cons
     return fail(VLG_ERR_UNSUPPORTED, "layout tile kernel: K / dtype not compiled in");
 }
 
-// Side stream + fork/join events of the calling thread (created once per thread and device).  Used to run the
-// label count next to the rgb strip kernel, which does not need it; works under stream capture too (the side
-// stream joins the capture through the fork event and is joined back before the layout kernel).
+// The rgb strip kernel with the gradient scales of `tc`: d(loss)/d(coords) (rgb part, nullable), the d(loss)/d(warped rgb)
+// staging for pass 2 (nullable) and one partial row per warp.
+static int launch_rgb_strips(const vlg_problem_t *prob, const TermCoeffs &tc, const void *src_rgb, const void *tgt_rgb,
+                             const float *coords, float *d_coords, float *d_out_rgb, bool need_grad, const WsLayout &L,
+                             char *ws, cudaStream_t st) {
+    RgbParams rp{};
+    rp.cc = make_cc(prob);
+    rp.N = (int)prob->N;
+    rp.strips = (int)((prob->W + kRS - 1) / kRS);
+    rp.total_rows = prob->N * rp.strips * prob->H;
+    rp.src_rgb = src_rgb; rp.tgt_rgb = tgt_rgb; rp.coords = coords;
+    rp.tc = tc;
+    rp.d_coords = d_coords;
+    rp.d_out_rgb = d_out_rgb;
+    rp.pitch = (int)L.pitch;
+    rp.partials = (float *)(ws + L.partials_rgb);
+    rp.hdr = (WsHeader *)(ws + L.header);
+    return prob->dtype == VLG_F32 ? launch_rgb<float>(rp, need_grad, st) : launch_rgb<__nv_bfloat16>(rp, need_grad, st);
+}
+
+// Side stream + fork/join events of the calling thread, one lane per device (created on first use).  Used to run the
+// label count next to the rgb strip kernel, which does not need it; works under stream capture too (the side stream
+// joins the capture through the fork event and is joined back before the layout kernel).
 struct SideLane {
-    int dev = -1;
     cudaStream_t s = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
 };
 static SideLane *side_lane() {
-    static thread_local SideLane lane;
+    static thread_local SideLane lanes[kMaxDevices];
     int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
-    if (lane.dev != dev) {
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) {
+        (void)cudaGetLastError();
+        return nullptr;
+    }
+    SideLane &lane = lanes[dev];
+    if (!lane.s) {
         SideLane nl;
         if (cudaStreamCreateWithFlags(&nl.s, cudaStreamNonBlocking) != cudaSuccess ||
             cudaEventCreateWithFlags(&nl.fork, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&nl.join, cudaEventDisableTiming) != cudaSuccess) {
+            if (nl.join) cudaEventDestroy(nl.join);
+            if (nl.fork) cudaEventDestroy(nl.fork);
+            if (nl.s) cudaStreamDestroy(nl.s);
             (void)cudaGetLastError();
             return nullptr;
         }
-        nl.dev = dev;
-        lane = nl;   // a lane of another device (if any) is left to the driver: a thread rarely changes device
+        lane = nl;
     }
     return &lane;
+}
+
+// The first launches of pass 1: count_valid_kernel (the CE divisor; when `count`) and `rgb()` (the rgb strip kernel;
+// when `has_rgb`).  The rgb kernel does not need the count, so the count runs beside it on the side lane, forked from
+// `st` and joined back into it on every path, before the layout kernel that `st` runs next.
+template <typename RgbLaunch>
+static int count_beside_rgb(const vlg_problem_t *prob, bool count, const int64_t *tgt_label, WsHeader *hdr, bool has_rgb,
+                            RgbLaunch rgb, cudaStream_t st) {
+    SideLane *lane = nullptr;
+    cudaStream_t cst = st;
+    if (count && has_rgb && (lane = side_lane()) != nullptr) {
+        if (cudaEventRecord(lane->fork, st) == cudaSuccess && cudaStreamWaitEvent(lane->s, lane->fork, 0) == cudaSuccess) cst = lane->s;
+        else lane = nullptr;
+    }
+    int rc = VLG_OK;
+    if (count) {
+        const int64_t P = prob->N * prob->H * prob->W;
+        const int blocks = (int)((P + 256 * 16 - 1) / (256 * 16));
+        count_valid_kernel<<<blocks < 1 ? 1 : blocks, 256, 0, cst>>>(tgt_label, P, prob->ignore_index, (int)prob->K,
+                                                                      prob->ce_class_weight, hdr);
+        rc = check_launch("count_valid_kernel");
+    }
+    const bool join_recorded = lane && cudaEventRecord(lane->join, lane->s) == cudaSuccess;
+    if (!rc && has_rgb) rc = rgb();
+    if (lane) {
+        if (!join_recorded) return rc ? rc : fail(VLG_ERR_CUDA, "side stream join record failed");
+        if (cudaStreamWaitEvent(st, lane->join, 0) != cudaSuccess && !rc) rc = fail(VLG_ERR_CUDA, "side stream join failed");
+    }
+    return rc;
 }
 
 static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, const void *src_layout,
@@ -750,26 +822,19 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     if (e != cudaSuccess) return fail(VLG_ERR_CUDA, "memset header: %s", cudaGetErrorString(e));
     const int64_t P = prob->N * prob->H * prob->W;
     const bool has_lay = src_layout && tgt_label;
-    const bool rgb_strips = warp && src_rgb && tgt_rgb && !(prob->flags & VLG_FLAG_TILE_RGB);
-    bool join_count = false;
-    SideLane *lane = nullptr;
-    if (has_lay) {
-        // the rgb strip kernel does not need the label count: fork it onto the side stream, join before the layout kernel
-        cudaStream_t cst = st;
-        if (rgb_strips && (lane = side_lane()) != nullptr && cudaEventRecord(lane->fork, st) == cudaSuccess &&
-            cudaStreamWaitEvent(lane->s, lane->fork, 0) == cudaSuccess) {
-            cst = lane->s;
-            join_count = true;
-        }
-        const int blocks = (int)((P + 256 * 16 - 1) / (256 * 16));
-        count_valid_kernel<<<blocks < 1 ? 1 : blocks, 256, 0, cst>>>(tgt_label, P, prob->ignore_index, (int)prob->K,
-                                                                      prob->ce_class_weight, hdr);
-        int rc = check_launch("count_valid_kernel");
-        if (join_count && cudaEventRecord(lane->join, lane->s) != cudaSuccess) return fail(VLG_ERR_CUDA, "side stream join record failed");
-        if (rc) return rc;
-    }
-    const double Ng = (double)(prob->global_N ? prob->global_N : prob->N);
-    const double H = (double)prob->H, W = (double)prob->W;
+    const bool rgb_strips = warp && src_rgb && tgt_rgb;
+    const TermCoeffs tc = make_terms(prob, warp);
+    // The rgb terms of a warped step run in the column-strip kernel, launched BEFORE the kernel that owns the layout / TV
+    // terms: it stores its part of d(loss)/d(coords); the layout kernel, which has issue slots to spare, loads that part
+    // one tile ahead, adds its own and performs the final reduction.
+    int rc = count_beside_rgb(prob, has_lay, tgt_label, hdr, rgb_strips, [&] {
+        tl_mark(kTlRgb0, st);
+        const int r = launch_rgb_strips(prob, tc, src_rgb, tgt_rgb, coords, need_grad ? d_coords : nullptr,
+                                        need_grad ? (float *)d_out_rgb : nullptr, need_grad, L, ws, st);
+        tl_mark(kTlRgb1, st);
+        return r;
+    }, st);
+    if (rc) return rc;
     Pass1Params pp{};
     pp.cc = make_cc(prob);
     pp.N = (int)prob->N;
@@ -778,17 +843,7 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     pp.src_rgb = src_rgb; pp.src_layout = src_layout; pp.coords = coords;
     pp.tgt_rgb = tgt_rgb; pp.label = tgt_label; pp.ignore_index = prob->ignore_index;
     pp.class_weight = prob->ce_class_weight;
-    pp.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
-    pp.c_l1 = (float)(prob->w_l1 / (Ng * 3 * H * W));
-    pp.c_gd = (float)(prob->w_gd / (Ng * 3 * H * W));
-    pp.c_ssim = (prob->H > 2 && prob->W > 2) ? (float)(prob->w_ssim / (2.0 * Ng * (H - 2) * (W - 2))) : 0.f;
-    pp.terms = prob->term_mask ? prob->term_mask : VLG_TERM_ALL;
-    if (!(prob->H > 2 && prob->W > 2)) pp.terms &= ~VLG_TERM_SSIM;
-    pp.do_tv = warp && prob->coord_mode == VLG_COORD_FLOW && (pp.terms & VLG_TERM_TV);
-    pp.c_tvh = prob->H > 1 ? (float)(prob->w_tv / (Ng * (H - 1) * W * 2)) : 0.f;
-    pp.c_tvw = prob->W > 1 ? (float)(prob->w_tv / (Ng * H * (W - 1) * 2)) : 0.f;
-    // a masked-out CE still runs its forward sum (the reduction drops it) but sends no gradient anywhere
-    pp.w_ce_over_scale = (pp.terms & VLG_TERM_CE) ? (float)(prob->w_ce * (double)prob->N / Ng) : 0.f;
+    pp.tc = tc;
     pp.need_grad = need_grad;
     pp.d_coords = d_coords; pp.d_out_rgb = d_out_rgb; pp.d_out_lay = d_out_lay;
     pp.out_argmax = out_argmax;
@@ -798,43 +853,14 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     pp.seg_cnt = (prob->flags & VLG_FLAG_FAR_WIDE) ? nullptr : (uint32_t *)(ws + L.seg_cnt);
     pp.far_list = (warp && d_out_lay && L.far_list) ? (int4 *)(ws + L.far_list) : nullptr;
     pp.flagged_list = (int *)(ws + L.flagged);
-    pp.red = make_reduce_params(prob, L, ws, fused_loss_out);
+    pp.red = make_reduce_params(prob, tc, L, ws, fused_loss_out);
     pp.hdr = hdr;
-    pp.flags = prob->flags;
-    pp.pitch = (int)L.pitch;
-    // tap records for pass 2: written by lay_tile_kernel on its way, by tap_records_kernel after the other organisations
+    pp.accum_dcoords = rgb_strips ? 1 : 0;
+    // tap records for pass 2: written by lay_tile_kernel on its way, by tap_records_kernel after pass1_kernel
     const bool want_records = warp && need_grad && d_out_lay != nullptr && L.rec_code != 0 && pass2_from_records(prob);
     bool records_done = false;
-    // The rgb terms run in the column-strip kernel, launched BEFORE the kernel that owns the layout / TV
-    // terms: it stores its part of d(loss)/d(coords) (and the label count); the layout kernel, which has
-    // issue slots to spare, loads that part one tile ahead, adds its own and performs the final reduction.
-    if (rgb_strips) {
-        RgbParams rp{};
-        rp.cc = pp.cc;
-        rp.N = (int)prob->N;
-        rp.strips = (int)((prob->W + kRS - 1) / kRS);
-        rp.total_rows = prob->N * rp.strips * prob->H;
-        rp.src_rgb = src_rgb; rp.tgt_rgb = tgt_rgb; rp.coords = coords;
-        rp.terms = pp.terms;
-        rp.c_l1 = (pp.terms & VLG_TERM_L1) ? pp.c_l1 : 0.f;
-        rp.c_gd = (pp.terms & VLG_TERM_GD) ? pp.c_gd : 0.f;
-        rp.c_ssim = (pp.terms & VLG_TERM_SSIM) ? pp.c_ssim : 0.f;
-        rp.d_coords = need_grad ? d_coords : nullptr;
-        rp.d_out_rgb = need_grad ? (float *)d_out_rgb : nullptr;
-        rp.pitch = (int)L.pitch;
-        rp.partials = (float *)(ws + L.partials_rgb);
-        rp.hdr = hdr;
-        tl_mark(kTlRgb0, st);
-        int rc0 = prob->dtype == VLG_F32 ? launch_rgb<float>(rp, need_grad, st) : launch_rgb<__nv_bfloat16>(rp, need_grad, st);
-        tl_mark(kTlRgb1, st);
-        if (rc0) return rc0;
-        pp.src_rgb = nullptr; pp.tgt_rgb = nullptr; pp.d_out_rgb = nullptr;
-        pp.accum_dcoords = 1;
-    }
-    if (join_count && cudaStreamWaitEvent(st, lane->join, 0) != cudaSuccess) return fail(VLG_ERR_CUDA, "side stream join failed");
-    int rc = VLG_OK;
     bool lay_done = false;
-    if (warp && has_lay && prob->K % 4 == 0 && !(prob->flags & (VLG_FLAG_NO_TMA | VLG_FLAG_TILE_LAYOUT))) {
+    if (warp && has_lay && prob->K % 4 == 0 && !(prob->flags & VLG_FLAG_NO_TMA)) {
         CUtensorMap row_map;
         bool px8 = false;
         if (make_window_map(prob, src_layout, &row_map, kTSW, kTSH, &px8)) {
@@ -843,9 +869,8 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
             lp.N = pp.N; lp.strips = pp.tiles_x; lp.tiles_y = pp.tiles_y;
             lp.total_rows = prob->N * (int64_t)lp.strips * prob->H;
             lp.src_layout = src_layout; lp.coords = coords; lp.label = tgt_label; lp.ignore_index = prob->ignore_index;
-            lp.class_weight = pp.class_weight; lp.weighted_denom = pp.weighted_denom;
-            lp.w_ce_over_scale = pp.w_ce_over_scale;
-            lp.c_tvh = pp.c_tvh; lp.c_tvw = pp.c_tvw; lp.do_tv = pp.do_tv;
+            lp.class_weight = pp.class_weight;
+            lp.tc = tc;
             lp.accum_dcoords = pp.accum_dcoords;
             lp.d_coords = need_grad ? d_coords : nullptr;
             lp.d_out_lay = need_grad ? (float *)d_out_lay : nullptr;
@@ -865,10 +890,7 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
         }
     }
     if (!lay_done) {
-        CUtensorMap lay_map;
-        pp.use_tma = (warp && has_lay && !(prob->flags & VLG_FLAG_NO_TMA) && make_layout_map(prob, src_layout, &lay_map)) ? 1 : 0;
-        if (!pp.use_tma) memset(&lay_map, 0, sizeof(lay_map));
-        rc = dispatch_pass1(prob, warp, pp, lay_map, L.n_blocks, st);
+        rc = dispatch_pass1(prob, warp, pp, st);
         if (rc) return rc;
     }
     if (want_records && !records_done) {
@@ -887,64 +909,26 @@ static int run_pass1_labels(const vlg_problem_t *prob, const void *src_rgb, cons
     char *ws = (char *)workspace;
     WsHeader *hdr = (WsHeader *)(ws + L.header);
     const int64_t P = prob->N * prob->H * prob->W;
-    const bool has_lay = src_label && tgt_label, has_rgb = src_rgb && tgt_rgb;
-    if (!has_lay) return fail(VLG_ERR_UNSUPPORTED, "the label-source op needs src_label / tgt_label (use vlg_pixel_loss_* for rgb-only criteria)");
+    const bool has_rgb = src_rgb && tgt_rgb;
+    if (!(src_label && tgt_label)) return fail(VLG_ERR_UNSUPPORTED, "the label-source op needs src_label / tgt_label (use vlg_pixel_loss_* for rgb-only criteria)");
     cudaError_t e = cudaMemsetAsync(hdr, 0, L.partials - L.header, st);
     if (e != cudaSuccess) return fail(VLG_ERR_CUDA, "memset header: %s", cudaGetErrorString(e));
     const bool need_grad = d_coords != nullptr;
-    bool join_count = false;
-    SideLane *lane = nullptr;
-    if (has_lay) {
-        cudaStream_t cst = st;
-        if (has_rgb && (lane = side_lane()) != nullptr && cudaEventRecord(lane->fork, st) == cudaSuccess &&
-            cudaStreamWaitEvent(lane->s, lane->fork, 0) == cudaSuccess) {
-            cst = lane->s;
-            join_count = true;
-        }
-        const int blocks = (int)((P + 256 * 16 - 1) / (256 * 16));
-        count_valid_kernel<<<blocks < 1 ? 1 : blocks, 256, 0, cst>>>(tgt_label, P, prob->ignore_index, (int)prob->K, prob->ce_class_weight, hdr);
-        int rc = check_launch("count_valid_kernel");
-        if (join_count && cudaEventRecord(lane->join, lane->s) != cudaSuccess) return fail(VLG_ERR_CUDA, "side stream join record failed");
-        if (rc) return rc;
-    }
-    const double Ng = (double)(prob->global_N ? prob->global_N : prob->N);
-    const double H = (double)prob->H, W = (double)prob->W;
-    uint32_t terms = prob->term_mask ? prob->term_mask : VLG_TERM_ALL;
-    if (!(prob->H > 2 && prob->W > 2)) terms &= ~VLG_TERM_SSIM;
-    const CoordCfg cc = make_cc(prob);
-    if (has_rgb) {
-        RgbParams rp{};
-        rp.cc = cc;
-        rp.N = (int)prob->N;
-        rp.strips = (int)((prob->W + kRS - 1) / kRS);
-        rp.total_rows = prob->N * rp.strips * prob->H;
-        rp.src_rgb = src_rgb; rp.tgt_rgb = tgt_rgb; rp.coords = coords;
-        rp.terms = terms;
-        rp.c_l1 = (terms & VLG_TERM_L1) ? (float)(prob->w_l1 / (Ng * 3 * H * W)) : 0.f;
-        rp.c_gd = (terms & VLG_TERM_GD) ? (float)(prob->w_gd / (Ng * 3 * H * W)) : 0.f;
-        rp.c_ssim = ((terms & VLG_TERM_SSIM) && prob->H > 2 && prob->W > 2) ? (float)(prob->w_ssim / (2.0 * Ng * (H - 2) * (W - 2))) : 0.f;
-        rp.d_coords = need_grad ? d_coords : nullptr;
-        rp.d_out_rgb = nullptr;            // sources are data: no pass 2, no staging
-        rp.pitch = (int)L.pitch;
-        rp.partials = (float *)(ws + L.partials_rgb);
-        rp.hdr = hdr;
-        int rc0 = prob->dtype == VLG_F32 ? launch_rgb<float>(rp, need_grad, st) : launch_rgb<__nv_bfloat16>(rp, need_grad, st);
-        if (rc0) return rc0;
-    }
-    if (join_count && cudaStreamWaitEvent(st, lane->join, 0) != cudaSuccess) return fail(VLG_ERR_CUDA, "side stream join failed");
+    const TermCoeffs tc = make_terms(prob, true);
+    // sources are data: no pass 2, no d(loss)/d(warped rgb) staging
+    int rc = count_beside_rgb(prob, true, tgt_label, hdr, has_rgb, [&] {
+        return launch_rgb_strips(prob, tc, src_rgb, tgt_rgb, coords, d_coords, nullptr, need_grad, L, ws, st);
+    }, st);
+    if (rc) return rc;
     LabParams lp{};
-    lp.cc = cc; lp.K = (int)prob->K; lp.P = P; lp.HW = prob->H * prob->W;
+    lp.cc = make_cc(prob); lp.K = (int)prob->K; lp.P = P; lp.HW = prob->H * prob->W;
     lp.src_label = src_label; lp.coords = (const float2 *)coords; lp.tgt_label = tgt_label; lp.ignore_index = prob->ignore_index;
     lp.class_weight = prob->ce_class_weight;
-    lp.weighted_denom = prob->ce_class_weight != nullptr && prob->ce_norm == VLG_CE_NORM_TORCH;
-    lp.w_ce_over_scale = (terms & VLG_TERM_CE) ? (float)(prob->w_ce * (double)prob->N / Ng) : 0.f;   // see run_pass1
-    lp.do_tv = prob->coord_mode == VLG_COORD_FLOW && (terms & VLG_TERM_TV);
-    lp.c_tvh = prob->H > 1 ? (float)(prob->w_tv / (Ng * (H - 1) * W * 2)) : 0.f;
-    lp.c_tvw = prob->W > 1 ? (float)(prob->w_tv / (Ng * H * (W - 1) * 2)) : 0.f;
+    lp.tc = tc;
     lp.accum_dcoords = has_rgb ? 1 : 0;
     lp.d_coords = d_coords; lp.out_argmax = out_argmax;
     lp.partials = (float *)(ws + L.partials_lay);
-    lp.red = make_reduce_params(prob, L, ws, loss_out);
+    lp.red = make_reduce_params(prob, tc, L, ws, loss_out);
     lp.hdr = hdr;
     int64_t blocks = (int64_t)sm_count() * 8;
     const int64_t max_blocks = (P + kLabThreads - 1) / kLabThreads;
@@ -1172,13 +1156,10 @@ int vlg_warp_bwd_src(const vlg_problem_t *prob, const float *coords, void *d_src
     pp.hdr = (WsHeader *)(ws + L.header);
     pp.tile_disp = (const float *)(ws + L.tile_disp);
     pp.HW = prob->H * prob->W;
-    const int64_t P = prob->N * pp.HW;
-    const size_t far_words = (size_t)P * (3 + prob->K);
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k)                                                                                       \
-    if (prob->K == k)                                                                              \
-        return prob->dtype == VLG_F32 ? launch_pass2<float, k>(pp, L.n_blocks, P, prob, far_words, st) \
-                                      : launch_pass2<__nv_bfloat16, k>(pp, L.n_blocks, P, prob, far_words, st);
+#define X(k)                                                                                                         \
+    if (prob->K == k)                                                                                                \
+        return prob->dtype == VLG_F32 ? launch_pass2<float, k>(pp, prob, st) : launch_pass2<__nv_bfloat16, k>(pp, prob, st);
     VLG_FOR_EACH_K(X)
 #undef X
     return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
@@ -1191,7 +1172,7 @@ int vlg_reduce_partials(const vlg_problem_t *prob, float *loss_out, void *worksp
     const WsLayout L = ws_layout(prob, 0);
     if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small");
     char *ws = (char *)workspace;
-    const ReduceParams rp = make_reduce_params(prob, L, ws, loss_out);
+    const ReduceParams rp = make_reduce_params(prob, make_terms(prob, true), L, ws, loss_out);
     reduce_partials_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(rp);
     return check_launch("reduce_partials_kernel");
 }

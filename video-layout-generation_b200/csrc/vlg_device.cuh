@@ -53,9 +53,23 @@ struct ReduceParams {
     double ce_scale;        // N_local/N_global
     float w_l1, w_gd, w_ssim, w_ce, w_tv;
     int weighted_denom;     // 1: CE divisor = hdr->ce_denom (class-weighted torch mean), 0: n_valid
-    int ce_on;              // VLG_TERM_CE is evaluated; 0: the CE slot reads 0 and stays out of the total
+    uint32_t terms;         // TermCoeffs::terms: the slot of a term whose bit is clear reads 0 and stays out of the total
     float *out;
 };
+
+// The loss terms a call evaluates and their gradient scales (upstream gradient 1.0), derived once on the host from the
+// problem (make_terms).  A coefficient is 0 when its term is off.
+struct TermCoeffs {
+    uint32_t terms;              // VLG_TERM_* bits in effect: term_mask (0 = all), SSIM cleared below 3x3, TV only for pixel flow
+    float c_l1, c_gd, c_ssim, c_tvh, c_tvw;
+    float w_ce_over_scale;       // w_ce * (N_local/N_global); divided by the CE divisor on the device
+    int weighted_denom;          // 1: CE divisor = hdr->ce_denom (class-weighted torch mean), 0: number of valid labels
+};
+
+// The CE divisor counted by count_valid_kernel, as the pass-1 kernels scale their CE gradient with it.
+__device__ __forceinline__ float ce_divisor(const TermCoeffs &tc, const WsHeader *hdr) {
+    return tc.weighted_denom ? (float)__ldcg(&hdr->ce_denom) : (float)__ldcg(&hdr->n_valid);
+}
 
 // Called by all NT threads of one CTA; `s` is 6*NT doubles of shared memory.
 template <int NT>
@@ -86,11 +100,12 @@ __device__ __forceinline__ void reduce_partials_block(const ReduceParams &p, dou
     }
     if (threadIdx.x == 0) {
         const double nv = (double)__ldcg(&p.hdr->n_valid);
-        const double l1 = s[0] * p.inv_numel_rgb, gd = s[NT] * p.inv_numel_rgb;
-        const double ssim = s[2 * NT] * p.inv_ssim;
+        const double l1 = (p.terms & VLG_TERM_L1) ? s[0] * p.inv_numel_rgb : 0.0;
+        const double gd = (p.terms & VLG_TERM_GD) ? s[NT] * p.inv_numel_rgb : 0.0;
+        const double ssim = (p.terms & VLG_TERM_SSIM) ? s[2 * NT] * p.inv_ssim : 0.0;
         const double cd = p.weighted_denom ? __ldcg(&p.hdr->ce_denom) : nv;
-        const double ce = (p.ce_on && cd > 0) ? s[3 * NT] / cd * p.ce_scale : 0.0;
-        const double tv = s[4 * NT] * p.inv_tvh + s[5 * NT] * p.inv_tvw;
+        const double ce = ((p.terms & VLG_TERM_CE) && cd > 0) ? s[3 * NT] / cd * p.ce_scale : 0.0;
+        const double tv = (p.terms & VLG_TERM_TV) ? s[4 * NT] * p.inv_tvh + s[5 * NT] * p.inv_tvw : 0.0;
         p.out[VLG_LOSS_L1] = (float)l1;
         p.out[VLG_LOSS_GD] = (float)gd;
         p.out[VLG_LOSS_SSIM] = (float)ssim;
@@ -489,17 +504,6 @@ __device__ __forceinline__ float dot2(const float (&g)[C], const float (&v)[C]) 
 __device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float lg2_approx(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-
-// ---------------------------------------------------------------- tuning builds: when do the CTAs of a persistent kernel start / finish?
-#ifdef VLG_PROFILE_TAIL
-__device__ __forceinline__ unsigned long long global_ns() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-// slots: [0] first start, [1] last start, [2] first end, [3] last end (prof must be pre-set to {~0, 0, ~0, 0})
-__device__ __forceinline__ void prof_mark(unsigned long long *slot4, bool end) {
-    const unsigned long long t = global_ns();
-    atomicMin(slot4 + (end ? 2 : 0), t);
-    atomicMax(slot4 + (end ? 3 : 1), t);
-}
-#endif
 
 // ---------------------------------------------------------------- tuning builds: when do the units of a persistent kernel finish?
 // (tools/tail_prof.py; -DVLG_PROFILE_TAIL)

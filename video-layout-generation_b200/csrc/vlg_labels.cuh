@@ -29,10 +29,7 @@ struct LabParams {
     const int64_t *tgt_label;
     int64_t ignore_index;
     const float *class_weight;
-    int weighted_denom;
-    float w_ce_over_scale;
-    float c_tvh, c_tvw;
-    int do_tv;
+    TermCoeffs tc;                 // w_ce_over_scale, weighted_denom, c_tvh, c_tvw; TV runs when terms has VLG_TERM_TV
     int accum_dcoords;             // d_coords already holds the rgb part (the rgb strip kernel ran before): add to it
     float *d_coords;               // nullable (validation)
     int64_t *out_argmax;           // nullable
@@ -52,8 +49,8 @@ __global__ void __launch_bounds__(kLabThreads) lab_pix_kernel(const LabParams p)
     const int H = cc.H, W = cc.W, K = p.K;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const float L2E = 1.4426950408889634f;
-    const float denom = GRAD ? (p.weighted_denom ? (float)__ldcg(&p.hdr->ce_denom) : (float)__ldcg(&p.hdr->n_valid)) : 1.0f;
-    const float ce_unit = GRAD ? p.w_ce_over_scale / denom : 0.f;
+    const float denom = GRAD ? ce_divisor(p.tc, p.hdr) : 1.0f;
+    const float ce_unit = GRAD ? p.tc.w_ce_over_scale / denom : 0.f;
     float s_ce = 0.f, s_tvh = 0.f, s_tvw = 0.f, m_disp = 0.f;
     bool bad = false;
 
@@ -141,12 +138,12 @@ __global__ void __launch_bounds__(kLabThreads) lab_pix_kernel(const LabParams p)
             gx = fmaf(t.mx, gix, gx);
             gy = fmaf(t.my, giy, gy);
         }
-        if (p.do_tv) {
+        if (p.tc.terms & VLG_TERM_TV) {
             const float2 *ci = p.coords + i;
             const bool hD = y + 1 < H, hU = y >= 1, hR = x + 1 < W, hL = x >= 1;
             const float2 fdn = hD ? __ldg(ci + W) : f, fup = hU ? __ldg(ci - W) : f;
             const float2 frt = hR ? __ldg(ci + 1) : f, flt = hL ? __ldg(ci - 1) : f;
-            const float cD = hD ? p.c_tvh : 0.f, cU = hU ? p.c_tvh : 0.f, cR = hR ? p.c_tvw : 0.f, cL = hL ? p.c_tvw : 0.f;
+            const float cD = hD ? p.tc.c_tvh : 0.f, cU = hU ? p.tc.c_tvh : 0.f, cR = hR ? p.tc.c_tvw : 0.f, cL = hL ? p.tc.c_tvw : 0.f;
             const float2 dd = make_float2(fdn.x - f.x, fdn.y - f.y), du = make_float2(f.x - fup.x, f.y - fup.y);
             const float2 dr = make_float2(frt.x - f.x, frt.y - f.y), dl = make_float2(f.x - flt.x, f.y - flt.y);
             s_tvh = fmaf(fabsf(dd.x) + fabsf(dd.y), hD ? 1.f : 0.f, s_tvh);

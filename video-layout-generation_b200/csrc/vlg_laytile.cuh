@@ -61,10 +61,7 @@ struct LayParams {
     const int64_t *label;
     int64_t ignore_index;
     const float *class_weight;
-    int weighted_denom;
-    float w_ce_over_scale;
-    float c_tvh, c_tvw;
-    int do_tv;
+    TermCoeffs tc;                 // w_ce_over_scale, weighted_denom, c_tvh, c_tvw; TV runs when terms has VLG_TERM_TV
     int accum_dcoords;             // d_coords already holds the rgb part (the rgb strip kernel ran before): add to it
     float *d_coords;               // nullable (validation)
     float *d_out_lay;              // [P][K] fp32 staging, nullable
@@ -128,8 +125,8 @@ __global__ void __launch_bounds__(kThreads, VLG_LAYTILE_MIN_BLOCKS) lay_tile_ker
     const float mx_c = (cc.coord_mode == VLG_COORD_FLOW) ? __fmul_rn(cc.Wm1, 0.5f) * cc.sx : __fmul_rn(cc.Wm1, 0.5f);
     const float my_c = (cc.coord_mode == VLG_COORD_FLOW) ? __fmul_rn(cc.Hm1, 0.5f) * cc.sy : __fmul_rn(cc.Hm1, 0.5f);
     const bool border = cc.padding == VLG_PAD_BORDER;
-    const float denom = GRAD ? (p.weighted_denom ? (float)__ldcg(&p.hdr->ce_denom) : (float)__ldcg(&p.hdr->n_valid)) : 1.0f;
-    const float ce_unit = GRAD ? p.w_ce_over_scale / denom : 0.f;
+    const float denom = GRAD ? ce_divisor(p.tc, p.hdr) : 1.0f;
+    const float ce_unit = GRAD ? p.tc.w_ce_over_scale / denom : 0.f;
     const float2 *coords_all = reinterpret_cast<const float2 *>(p.coords);
     const T *src_all = reinterpret_cast<const T *>(p.src_layout);
 
@@ -164,15 +161,15 @@ __global__ void __launch_bounds__(kThreads, VLG_LAYTILE_MIN_BLOCKS) lay_tile_ker
         return i < nt ? __ldg(coords_all + px_index(g, wid, lane)) : make_float2(0.f, 0.f);
     };
     auto load_label = [&](int i, const TileGeo &g) -> int64_t { return i < nt ? __ldg(p.label + px_index(g, wid, lane)) : (int64_t)0; };
-    // halo of the flow block: threads 0..83 own one halo cell each (top row, bottom row, left / right column)
+    // halo of the flow block (TV only): threads 0..83 own one halo cell each (top row, bottom row, left / right column)
     int hy = 0, hx = 0;                 // halo cell of this thread, relative to the tile origin
-    const bool has_halo = p.do_tv && tid < 2 * kFW + 2 * kTH;
+    const bool has_halo = tid < 2 * kFW + 2 * kTH;
     if (tid < kFW) { hy = -1; hx = tid - 1; }
     else if (tid < 2 * kFW) { hy = kTH; hx = tid - kFW - 1; }
     else if (tid < 2 * kFW + kTH) { hy = tid - 2 * kFW; hx = -1; }
     else { hy = tid - 2 * kFW - kTH; hx = kTW; }
     auto load_halo = [&](int i, const TileGeo &g) -> float2 {
-        return (i < nt && has_halo) ? __ldg(coords_all + px_index(g, hy, hx)) : make_float2(0.f, 0.f);
+        return (i < nt && has_halo && (p.tc.terms & VLG_TERM_TV)) ? __ldg(coords_all + px_index(g, hy, hx)) : make_float2(0.f, 0.f);
     };
     // sampling position of this thread's pixel + its contribution to the tile's window origin
     // (mean tap displacement of the tile: robust against a few outliers)
@@ -190,7 +187,7 @@ __global__ void __launch_bounds__(kThreads, VLG_LAYTILE_MIN_BLOCKS) lay_tile_ker
         return xy;
     };
     auto publish_flow = [&](int i, float2 fl, float2 fh, int buf) {
-        if (i >= nt || !p.do_tv) return;
+        if (i >= nt || !(p.tc.terms & VLG_TERM_TV)) return;
         sm.flow[buf][(wid + 1) * kFW + lane + 1] = fl;
         if (has_halo) sm.flow[buf][(hy + 1) * kFW + hx + 1] = fh;
     };
@@ -412,11 +409,11 @@ __global__ void __launch_bounds__(kThreads, VLG_LAYTILE_MIN_BLOCKS) lay_tile_ker
 
         // ---- coordinate gradient: layout part + TV ----
         float gx = fmaf(tp.mx, gix, dc.x), gy = fmaf(tp.my, giy, dc.y);
-        if (p.do_tv) {
+        if (p.tc.terms & VLG_TERM_TV) {
             const float2 *fc = &sm.flow[i & 3][(wid + 1) * kFW + lane + 1];
             const float2 f = f0, fdn = fc[kFW], fup = fc[-kFW], frt = fc[1], flt = fc[-1];
-            const float cD = (inside && y + 1 < H) ? p.c_tvh : 0.f, cU = (inside && y >= 1) ? p.c_tvh : 0.f;
-            const float cR = (inside && x + 1 < W) ? p.c_tvw : 0.f, cL = (inside && x >= 1) ? p.c_tvw : 0.f;
+            const float cD = (inside && y + 1 < H) ? p.tc.c_tvh : 0.f, cU = (inside && y >= 1) ? p.tc.c_tvh : 0.f;
+            const float cR = (inside && x + 1 < W) ? p.tc.c_tvw : 0.f, cL = (inside && x >= 1) ? p.tc.c_tvw : 0.f;
             const float2 dd = make_float2(fdn.x - f.x, fdn.y - f.y), du = make_float2(f.x - fup.x, f.y - fup.y);
             const float2 dr = make_float2(frt.x - f.x, frt.y - f.y), dl = make_float2(f.x - flt.x, f.y - flt.y);
             s_tvh = fmaf(fabsf(dd.x) + fabsf(dd.y), (inside && y + 1 < H) ? 1.f : 0.f, s_tvh);

@@ -1,5 +1,7 @@
 // vlg_pass1.cuh -- pass 1 of the fused op: warp + every per-pixel loss term + d(loss)/d(warped)
 // + d(loss)/d(coords) in ONE kernel, one CTA per 32x8 output tile (grid = tiles_x x tiles_y x N).
+// It evaluates the un-warped criteria (vlg_pixel_loss_*, rgb and layout) and, for a warped step, the layout
+// and TV terms when lay_tile_kernel cannot take them; the rgb terms of a warped step run in rgb_strip_kernel.
 //
 // Loss definitions followed (reference gongaa/video-layout-generation):
 //   L1          src/trainer.py:130,248      mean |a-b| over N*3*H*W, sign(0)=0
@@ -13,7 +15,7 @@
 // The kernel is issue-bound, not HBM-bound (profiles/): everything below is organised to spend
 // few instructions per pixel.  Phases of one CTA (256 threads, tile 32x8, rgb halo 2):
 //   0a  base-grid coordinates of the tile's rows/columns -> smem (one IEEE division each)
-//   0b  rgb over tile+halo: sampling coordinates, 4-tap gather of src_rgb, target -> smem;
+//   0b  over tile+halo: rgb (given) and target -> smem, or (WARP) the coordinates -> smem and the
 //       bounding box of the layout taps of the tile's own pixels (integer smem atomics)
 //   1   cp.async the source-layout bounding box into smem row by row (zero-filled outside the
 //       image), and meanwhile evaluate the 3x3 SSIM windows (runs of 5 share their column sums,
@@ -32,24 +34,18 @@ struct Pass1Params {
     CoordCfg cc;
     int N;
     int tiles_x, tiles_y;
-    const void *src_rgb, *src_layout;  // WARP: sources.  !WARP: `output` rgb / logits themselves
+    const void *src_rgb, *src_layout;  // WARP: source layout (src_rgb unused).  !WARP: `output` rgb / logits themselves
     const float *coords;
     const void *tgt_rgb;
     const int64_t *label;
     int64_t ignore_index;
     const float *class_weight;   // per-class CE weights (K floats) or NULL
-    int weighted_denom;          // 1: CE divisor = hdr->ce_denom, 0: number of valid labels
-    // gradient scales (upstream grad 1.0), host-computed in double
-    float c_l1, c_gd, c_ssim, c_tvh, c_tvw;
-    float w_ce_over_scale;  // w_ce * (N_local/N_global); divided by n_valid on the device
+    TermCoeffs tc;
     int need_grad;          // compute gradients at all
-    int do_tv;
-    uint32_t terms;         // VLG_TERM_* bits to evaluate
     // outputs
     float *d_coords;        // WARP && need_grad
-    void *d_out_rgb;        // WARP: fp32 staging, rows of `pitch` pixels (nullable). !WARP: user tensor of type T (nullable)
+    void *d_out_rgb;        // !WARP: user tensor of type T (nullable)
     void *d_out_lay;
-    int pitch;              // row pitch (pixels) of the WARP d_out_rgb staging
     int64_t *out_argmax;    // nullable
     float *partials;        // [n_blocks][kPartialSlots]
     float *tile_disp;       // [n_blocks] max displacement among the tile's NEAR output pixels (WARP)
@@ -59,8 +55,6 @@ struct Pass1Params {
     int *flagged_list;      // [n_blocks] compacted ids of the flagged source tiles
     ReduceParams red;       // red.out != NULL: the last CTA also performs the final reduction
     WsHeader *hdr;
-    uint32_t flags;
-    int use_tma;            // the layout window is staged by one cp.async.bulk.tensor per CTA
     int accum_dcoords;      // d_coords already holds the rgb part (written by rgb_strip_kernel): add to it
 };
 
@@ -92,7 +86,6 @@ struct Pass1Smem {
     float red[kThreads / 32][kPartialSlots];
     float redmax[kThreads / 32][4];
     int bbox[4];            // min x0, min y0, max x0, max y0 of the tile's own taps
-    alignas(8) uint64_t tma_bar;           // mbarrier the TMA load of the layout window completes on
     alignas(128) T stage[kSH * kSW * K];   // staged source-layout window
 };
 static_assert(sizeof(float2) * 3 * kRN + sizeof(float) * 9 * kWN >= 6 * 256 * sizeof(double),
@@ -223,7 +216,7 @@ __device__ __forceinline__ float tap_global(const T *img, int C, int c, int y, i
 }
 
 template <typename T, int K, bool WARP>
-__global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(const Pass1Params p, const __grid_constant__ CUtensorMap lay_map) {
+__global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(const Pass1Params p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Pass1Smem<T, K> &sm = *reinterpret_cast<Pass1Smem<T, K> *>(smem_raw);
     const CoordCfg &cc = p.cc;
@@ -235,7 +228,8 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
     const int ty0 = blockIdx.y * kTH, tx0 = blockIdx.x * kTW;
     const int64_t img_px = (int64_t)n * H * W;
 
-    const bool has_rgb = p.src_rgb != nullptr && p.tgt_rgb != nullptr;
+    // a warped step evaluates its rgb terms in rgb_strip_kernel
+    const bool has_rgb = !WARP && p.src_rgb != nullptr && p.tgt_rgb != nullptr;
     const bool has_lay = p.src_layout != nullptr && p.label != nullptr;
     const T *src_rgb = has_rgb ? reinterpret_cast<const T *>(p.src_rgb) + img_px * 3 : nullptr;
     const T *tgt_rgb = has_rgb ? reinterpret_cast<const T *>(p.tgt_rgb) + img_px * 3 : nullptr;
@@ -259,7 +253,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
             if (p.class_weight && lab_pre >= 0 && lab_pre < K) wl_pre = __ldg(p.class_weight + lab_pre);
         }
         if (has_lay && p.need_grad)
-            denom_pre = p.weighted_denom ? (float)__ldcg(&p.hdr->ce_denom) : (float)__ldcg(&p.hdr->n_valid);
+            denom_pre = ce_divisor(p.tc, p.hdr);
     }
 
     // ---------------- phase 0a: base grid of the region's rows / columns ----------------
@@ -267,75 +261,12 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
         if (tid < kRW) sm.bx[tid] = base_coord(tx0 - kHalo + tid, cc.Wm1);
         else if (tid >= 64 && tid < 64 + kRH) sm.by[tid - 64] = base_coord(ty0 - kHalo + tid - 64, cc.Hm1);
         if (tid == 128) { sm.bbox[0] = 1 << 30; sm.bbox[1] = 1 << 30; sm.bbox[2] = -(1 << 30); sm.bbox[3] = -(1 << 30); }
-        if (tid == 160 && p.use_tma) mbar_init(&sm.tma_bar, 1);
         // (the barrier that publishes the table sits in phase 0b, after the coords loads were issued)
     }
 
     // ---------------- phase 0b: coordinates + rgb over the tile + halo ----------------
     {
         int bx0 = 1 << 30, by0 = 1 << 30, bx1 = -(1 << 30), by1 = -(1 << 30);
-        constexpr int kIt = (kRN + kThreads - 1) / kThreads;
-        if (WARP && has_rgb) {
-            // Branch-free, software-pipelined form of the generic loop below: every address is clamped
-            // into the image so that all loads are unconditional and the loads of BOTH region pixels
-            // of a thread are in flight together (coords -> 12 tap channels + 3 target channels);
-            // out-of-image taps are zeroed by a select, exactly like the predicated gather.
-            bool inside[kIt];
-            int64_t oc[kIt];
-            int rxs[kIt], rys[kIt];
-            float2 fl[kIt];
-#pragma unroll
-            for (int it = 0; it < kIt; ++it) {
-                const int q = min(tid + it * kThreads, kRN - 1);
-                const int ry = q / kRW, rx = q - ry * kRW;
-                const int y = ty0 - kHalo + ry, x = tx0 - kHalo + rx;
-                inside[it] = tid + it * kThreads < kRN && y >= 0 && y < H && x >= 0 && x < W;
-                oc[it] = (int64_t)min(max(y, 0), H - 1) * W + min(max(x, 0), W - 1);
-                rxs[it] = rx; rys[it] = ry;
-                fl[it] = __ldg(coords + oc[it]);
-            }
-            __syncthreads();   // base-grid table ready; the coords loads above are already in flight
-            Taps tp[kIt];
-            float v[kIt][4][3], tb[kIt][3];
-#pragma unroll
-            for (int it = 0; it < kIt; ++it) {
-                float mx, my;
-                const float2 xy = source_xy(cc, fl[it], sm.bx[rxs[it]], sm.by[rys[it]], mx, my);
-                tp[it] = taps_from_xy(cc, xy, mx, my);
-                const bool own = rys[it] >= kHalo && rys[it] < kHalo + kTH && rxs[it] >= kHalo && rxs[it] < kHalo + kTW;
-                if (own && has_lay && inside[it]) {
-                    bx0 = min(bx0, tp[it].x0); bx1 = max(bx1, tp[it].x0);
-                    by0 = min(by0, tp[it].y0); by1 = max(by1, tp[it].y0);
-                }
-                const int x0c = min(max(tp[it].x0, 0), W - 1), x1c = min(max(tp[it].x0 + 1, 0), W - 1);
-                const int y0c = min(max(tp[it].y0, 0), H - 1), y1c = min(max(tp[it].y0 + 1, 0), H - 1);
-                load_px<T, 3>(src_rgb + ((int64_t)y0c * W + x0c) * 3, v[it][0]);
-                load_px<T, 3>(src_rgb + ((int64_t)y0c * W + x1c) * 3, v[it][1]);
-                load_px<T, 3>(src_rgb + ((int64_t)y1c * W + x0c) * 3, v[it][2]);
-                load_px<T, 3>(src_rgb + ((int64_t)y1c * W + x1c) * 3, v[it][3]);
-                load_px<T, 3>(tgt_rgb + oc[it] * 3, tb[it]);
-            }
-#pragma unroll
-            for (int it = 0; it < kIt; ++it) {
-                const Taps &t = tp[it];
-                const bool xin0 = t.x0 >= 0 && t.x0 < W, xin1 = t.x0 + 1 >= 0 && t.x0 + 1 < W;
-                const bool yin0 = t.y0 >= 0 && t.y0 < H, yin1 = t.y0 + 1 >= 0 && t.y0 + 1 < H;
-                const int q = tid + it * kThreads;
-                if (q < kRN) {
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {
-                        float acc = __fmul_rn(yin0 && xin0 ? v[it][0][c] : 0.0f, t.nw);
-                        acc = __fmaf_rn(yin0 && xin1 ? v[it][1][c] : 0.0f, t.ne, acc);
-                        acc = __fmaf_rn(yin1 && xin0 ? v[it][2][c] : 0.0f, t.sw, acc);
-                        acc = __fmaf_rn(yin1 && xin1 ? v[it][3][c] : 0.0f, t.se, acc);
-                        sm.ab[c][q] = inside[it] ? make_float2(acc, tb[it][c]) : make_float2(0.f, 0.f);
-                    }
-#if VLG_P1_FLOW_IN_SMEM
-                    sm.flow[q] = inside[it] ? fl[it] : make_float2(0.f, 0.f);
-#endif
-                }
-            }
-        } else {
         if (WARP) __syncthreads();   // base-grid table ready
 #pragma unroll
         for (int it = 0; it < (kRN + kThreads - 1) / kThreads; ++it) {
@@ -351,10 +282,6 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
                         float mx, my;
                         fl = __ldg(coords + o);
                         const float2 xy = source_xy(cc, fl, sm.bx[rx], sm.by[ry], mx, my);
-                        if (has_rgb) {
-                            const Taps t = taps_from_xy(cc, xy, mx, my);
-                            gather_px<T, 3>(src_rgb, cc, t, a);
-                        }
                         const bool own = ry >= kHalo && ry < kHalo + kTH && rx >= kHalo && rx < kHalo + kTW;
                         if (own && has_lay) {
                             const int x0 = (int)fminf(fmaxf(floorf(xy.x), -4.0f), (float)W + 4.0f);
@@ -375,7 +302,6 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
                 if (WARP) sm.flow[q] = fl;
 #endif
             }
-        }
         }
         if (WARP && has_lay) {
             bx0 = __reduce_min_sync(0xffffffffu, bx0); by0 = __reduce_min_sync(0xffffffffu, by0);
@@ -398,14 +324,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
         sh = min(kSH, sm.bbox[3] + 2 - oy);
         constexpr int PXB = K * (int)sizeof(T);
         constexpr int VB = vec_bytes(PXB);
-        if (p.use_tma) {
-            // one elected thread: the full kSW x kSH window at (ox, oy) of image n, zero-filled outside
-            sw = kSW; sh = kSH;
-            if (tid == 0) {
-                mbar_expect_tx(&sm.tma_bar, (unsigned)(kSH * kSW * PXB));
-                tma_load_4d(sm.stage, &lay_map, &sm.tma_bar, 0, ox, oy, n);
-            }
-        } else if (sw > 0 && sh > 0) {
+        if (sw > 0 && sh > 0) {
             const int xa = min(max(0, ox), ox + sw), xb = max(min(ox + sw, W), xa);   // in-image columns [xa, xb)
             for (int ry = wid; ry < sh; ry += kThreads / 32) {
                 const int y = oy + ry;
@@ -433,7 +352,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
     }
 
     // ---------------- phase 1b: SSIM windows, runs of kSegW along x ----------------
-    if (has_rgb && (p.terms & VLG_TERM_SSIM)) {
+    if (has_rgb && (p.tc.terms & VLG_TERM_SSIM)) {
         if (tid < kSegs * kWH * 3) {
             const int c = tid / (kSegs * kWH);
             const int r2 = tid - c * (kSegs * kWH);
@@ -460,7 +379,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
             const bool row_ok = i >= 0 && i + 2 < H;
             const float inv9 = 1.0f / 9.0f, C1 = 1e-4f, C2 = 9e-4f;
             const float2 inv9_2 = make_float2(inv9, inv9);
-            const float kk = -p.c_ssim * (2.0f / 9.0f);
+            const float kk = -p.tc.c_ssim * (2.0f / 9.0f);
 #pragma unroll
             for (int w = 0; w < kSegW; ++w) {
                 if (w < nwin) {
@@ -494,10 +413,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
             }
         }
     }
-    if (WARP && has_lay) {
-        if (p.use_tma) mbar_wait(&sm.tma_bar, 0);
-        else cp_async_commit_wait_all();
-    }
+    if (WARP && has_lay) cp_async_commit_wait_all();
     __syncthreads();
 
     // ---------------- phase 2: own pixel ----------------
@@ -540,37 +456,37 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
                 const float a = ab0.x, b = ab0.y;
                 const float d = a - b;
                 float g = 0.f;
-                if (p.terms & VLG_TERM_L1) {
+                if (p.tc.terms & VLG_TERM_L1) {
                     s_l1 += fabsf(d);
-                    g = signed_c1(p.c_l1, d);
+                    g = signed_c1(p.tc.c_l1, d);
                 }
-                if (p.terms & VLG_TERM_GD) {
+                if (p.tc.terms & VLG_TERM_GD) {
                     // vertical pairs (reference `xloss`, src/loss.py:21-22): (y -> y+1) owned here
                     if (y + 1 < H) {
                         const float2 dv = __fadd2_rn(sm.ab[c][q0 + kRW], make_float2(-a, -b));
                         const float tt = fabsf(dv.x) - fabsf(dv.y);
                         s_gd += fabsf(tt);
-                        g -= signed_c(p.c_gd, tt, dv.x);
+                        g -= signed_c(p.tc.c_gd, tt, dv.x);
                     }
                     if (y >= 1) {
                         const float2 v = sm.ab[c][q0 - kRW];
                         const float da = a - v.x;
-                        g += signed_c(p.c_gd, fabsf(da) - fabsf(b - v.y), da);
+                        g += signed_c(p.tc.c_gd, fabsf(da) - fabsf(b - v.y), da);
                     }
                     // horizontal pairs (reference `yloss`, src/loss.py:23-24)
                     if (x + 1 < W) {
                         const float2 dv = __fadd2_rn(sm.ab[c][q0 + 1], make_float2(-a, -b));
                         const float tt = fabsf(dv.x) - fabsf(dv.y);
                         s_gd += fabsf(tt);
-                        g -= signed_c(p.c_gd, tt, dv.x);
+                        g -= signed_c(p.tc.c_gd, tt, dv.x);
                     }
                     if (x >= 1) {
                         const float2 v = sm.ab[c][q0 - 1];
                         const float da = a - v.x;
-                        g += signed_c(p.c_gd, fabsf(da) - fabsf(b - v.y), da);
+                        g += signed_c(p.tc.c_gd, fabsf(da) - fabsf(b - v.y), da);
                     }
                 }
-                if (p.need_grad && (p.terms & VLG_TERM_SSIM)) {
+                if (p.need_grad && (p.tc.terms & VLG_TERM_SSIM)) {
                     // SSIM adjoint: the <=9 windows whose footprint contains this pixel
                     float2 sAB = make_float2(0.f, 0.f);
                     float sC = 0.f;
@@ -588,34 +504,8 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
                 dr[c] = g;
                 m_grad = fmaxf(m_grad, fabsf(g));
             }
-            if (p.need_grad) {
-                if (WARP) {
-                    {   // branch-free form of coord_grad_px: clamped addresses, all 12 loads in flight together
-                        const int x0c = min(max(t.x0, 0), W - 1), x1c = min(max(t.x0 + 1, 0), W - 1);
-                        const int y0c = min(max(t.y0, 0), H - 1), y1c = min(max(t.y0 + 1, 0), H - 1);
-                        float tv[4][3];
-                        load_px<T, 3>(src_rgb + ((int64_t)y0c * W + x0c) * 3, tv[0]);
-                        load_px<T, 3>(src_rgb + ((int64_t)y0c * W + x1c) * 3, tv[1]);
-                        load_px<T, 3>(src_rgb + ((int64_t)y1c * W + x0c) * 3, tv[2]);
-                        load_px<T, 3>(src_rgb + ((int64_t)y1c * W + x1c) * 3, tv[3]);
-                        const bool xin0 = t.x0 >= 0 && t.x0 < W, xin1 = t.x0 + 1 >= 0 && t.x0 + 1 < W;
-                        const bool yin0 = t.y0 >= 0 && t.y0 < H, yin1 = t.y0 + 1 >= 0 && t.y0 + 1 < H;
-                        const bool tin[4] = {yin0 && xin0, yin0 && xin1, yin1 && xin0, yin1 && xin1};
-                        float dt4[4];
-#pragma unroll
-                        for (int k4 = 0; k4 < 4; ++k4) {
-                            const float s3 = fmaf(dr[2], tv[k4][2], fmaf(dr[1], tv[k4][1], dr[0] * tv[k4][0]));
-                            dt4[k4] = tin[k4] ? s3 : 0.0f;
-                        }
-                        const float wx1 = t.ix - t.fx0, wx0 = (t.fx0 + 1.0f) - t.ix;
-                        const float wy1 = t.iy - t.fy0, wy0 = (t.fy0 + 1.0f) - t.iy;
-                        gix += (dt4[1] - dt4[0]) * wy0 + (dt4[3] - dt4[2]) * wy1;
-                        giy += (dt4[2] - dt4[0]) * wx0 + (dt4[3] - dt4[1]) * wx1;
-                    }
-                    if (p.d_out_rgb) store_px<float, 3>(reinterpret_cast<float *>(p.d_out_rgb) + (((int64_t)n * H + y) * p.pitch + x) * 3, dr);
-                } else if (p.d_out_rgb) {
-                    store_px<T, 3>(reinterpret_cast<T *>(p.d_out_rgb) + (img_px + o) * 3, dr);
-                }
+            if (p.need_grad && p.d_out_rgb) {
+                store_px<T, 3>(reinterpret_cast<T *>(p.d_out_rgb) + (img_px + o) * 3, dr);
             }
         }
 
@@ -671,7 +561,7 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
             }
             if (lab_ok) s_ce += wl_pre * (fmaf(lg2_approx(se), 0.6931471805599453f, m) - zl);
             if (p.need_grad) {
-                const float cce = lab_ok ? p.w_ce_over_scale * wl_pre / denom_pre : 0.0f;
+                const float cce = lab_ok ? p.tc.w_ce_over_scale * wl_pre / denom_pre : 0.0f;
                 const float inv = cce / se;
                 // d/dz_k = cce * (softmax_k - [k == label]); the one-hot part is applied to the label
                 // channel alone (a scalar fix-up store / a rank-1 term of the coordinate gradient)
@@ -714,29 +604,29 @@ __global__ void __launch_bounds__(kThreads, VLG_P1_MIN_BLOCKS) pass1_kernel(cons
 
         if (WARP) {
             float gx = fmaf(t.mx, gix, dc_pre.x), gy = fmaf(t.my, giy, dc_pre.y);
-            if (p.do_tv) {
+            if (p.tc.terms & VLG_TERM_TV) {
                 const float2 f = VLG_FLOW_AT(0, 0);
                 if (y + 1 < H) {
                     const float2 df = __fadd2_rn(VLG_FLOW_AT(kRW, W), make_float2(-f.x, -f.y));
                     s_tvh += fabsf(df.x) + fabsf(df.y);
-                    gx -= signed_c1(p.c_tvh, df.x);
-                    gy -= signed_c1(p.c_tvh, df.y);
+                    gx -= signed_c1(p.tc.c_tvh, df.x);
+                    gy -= signed_c1(p.tc.c_tvh, df.y);
                 }
                 if (y >= 1) {
                     const float2 f1 = VLG_FLOW_AT(-kRW, -W);
-                    gx += signed_c1(p.c_tvh, f.x - f1.x);
-                    gy += signed_c1(p.c_tvh, f.y - f1.y);
+                    gx += signed_c1(p.tc.c_tvh, f.x - f1.x);
+                    gy += signed_c1(p.tc.c_tvh, f.y - f1.y);
                 }
                 if (x + 1 < W) {
                     const float2 df = __fadd2_rn(VLG_FLOW_AT(1, 1), make_float2(-f.x, -f.y));
                     s_tvw += fabsf(df.x) + fabsf(df.y);
-                    gx -= signed_c1(p.c_tvw, df.x);
-                    gy -= signed_c1(p.c_tvw, df.y);
+                    gx -= signed_c1(p.tc.c_tvw, df.x);
+                    gy -= signed_c1(p.tc.c_tvw, df.y);
                 }
                 if (x >= 1) {
                     const float2 f1 = VLG_FLOW_AT(-1, -1);
-                    gx += signed_c1(p.c_tvw, f.x - f1.x);
-                    gy += signed_c1(p.c_tvw, f.y - f1.y);
+                    gx += signed_c1(p.tc.c_tvw, f.x - f1.x);
+                    gy += signed_c1(p.tc.c_tvw, f.y - f1.y);
                 }
             }
             if (p.need_grad && p.d_coords)

@@ -45,8 +45,7 @@ struct RgbParams {
     int64_t chunk;                  // rows per warp (contiguous in (n, strip, y) order)
     const void *src_rgb, *tgt_rgb;
     const float *coords;
-    float c_l1, c_gd, c_ssim;       // gradient scales (0 when the term is masked off)
-    uint32_t terms;
+    TermCoeffs tc;                  // c_l1, c_gd, c_ssim: the rgb gradient scales
     float *d_coords;                // [P][2] rgb part of d(loss)/d(coords); the layout kernel that follows adds its own (nullable)
     float *d_out_rgb;               // [N][H][pitch][3] fp32 staging for pass 2 (nullable)
     int pitch;
@@ -120,7 +119,7 @@ __global__ void __launch_bounds__(kRgbThreads, VLG_RGB_MIN_BLOCKS) rgb_strip_ker
 #endif
 
     const float inv9 = 1.0f / 9.0f, C1 = 1e-4f, C2 = 9e-4f;
-    const float kk = -p.c_ssim * (2.0f / 9.0f);
+    const float kk = -p.tc.c_ssim * (2.0f / 9.0f);
 
     while (rho < rho_end) {
         // ---- one segment: rows [ya, yb) of strip s of image n ----
@@ -135,8 +134,8 @@ __global__ void __launch_bounds__(kRgbThreads, VLG_RGB_MIN_BLOCKS) rgb_strip_ker
         const bool out_lane = lane >= 2 && lane < 30 && x < W;
         const int xc = min(max(x, 0), W - 1);
         const float bxv = base_coord(xc, cc.Wm1);
-        const float cR = (col_ok && x + 1 < W) ? p.c_gd : 0.f;      // pair (x, x+1) exists
-        const float cV = col_ok ? p.c_gd : 0.f;
+        const float cR = (col_ok && x + 1 < W) ? p.tc.c_gd : 0.f;   // pair (x, x+1) exists
+        const float cV = col_ok ? p.tc.c_gd : 0.f;
         const float mR = (out_lane && x + 1 < W) ? 1.f : 0.f;       // this lane counts the pair (x, x+1)
         const bool win_x = x >= 1 && x <= W - 2;                    // a 3x3 window can be centred on column x
         const int64_t img = (int64_t)n * H * W;
@@ -225,7 +224,7 @@ __global__ void __launch_bounds__(kRgbThreads, VLG_RGB_MIN_BLOCKS) rgb_strip_ker
                 // L1
                 const float d = a - b;
                 s_l1 = fmaf(fabsf(d), mo0, s_l1);
-                float g = signed_c1(p.c_l1, d);
+                float g = signed_c1(p.tc.c_l1, d);
                 // GD along W (reference `yloss`, src/loss.py:23-24): pairs (x, x+1) and (x-1, x)
                 {   // each lane evaluates its pair (x, x+1) once; the right neighbour receives the gradient by a shuffle
                     const float da = ar - a, tt = fabsf(da) - fabsf(br - b);
@@ -322,16 +321,17 @@ __global__ void __launch_bounds__(kRgbThreads, VLG_RGB_MIN_BLOCKS) rgb_strip_ker
         for (; t <= t_last; ++t) row_step(std::false_type{}, t);
     }
 
-    // ---- per-warp partial sums (fixed order: the final reduction walks the rows by index) ----
+    // ---- per-warp partial sums (fixed order: the final reduction walks the rows by index; it also reads the slot of a
+    // masked-off term as 0) ----
     s_l1 = warp_sum(s_l1);
     s_gd = warp_sum(s_gd);
     s_ssim = warp_sum(s_ssim);
     m_grad = warp_max(m_grad);
     if (lane == 0) {
         float4 o;
-        o.x = (p.terms & VLG_TERM_L1) ? s_l1 : 0.f;
-        o.y = (p.terms & VLG_TERM_GD) ? s_gd : 0.f;
-        o.z = (p.terms & VLG_TERM_SSIM) ? s_ssim : 0.f;
+        o.x = s_l1;
+        o.y = s_gd;
+        o.z = s_ssim;
         o.w = 0.f;
 #ifdef VLG_PROFILE_TAIL
         o.w = __uint_as_float(prof_stamp());     // where and when this warp finished

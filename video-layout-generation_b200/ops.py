@@ -39,9 +39,6 @@ class WarpLossConfig:
     global_batch: int = 0                 # data-parallel: divisor batch (0 = local batch)
     assume_near: bool = False             # caller asserts |flow| < NEAR_RADIUS: skip far-path launches
     use_tma: bool = True                  # stage source layout rows / windows with TMA tensor maps when possible
-    tile_kernels: bool = False            # evaluate ALL of pass 1 in the first (non-persistent) 32x8 tile kernel
-    layout_kernel: str = "tile2"          # layout half of pass 1: 'tile2' persistent double-buffered tile kernel (default),
-                                          # 'tile' first tile kernel
     pass2_records: bool = True            # pass 2 gathers from the tap records pass 1 wrote (all staging by TMA);
                                           # False: it re-derives them from the coordinates (first pass-2 kernel)
     far_packed: bool = True               # far path packs two 32-bit lanes per 64-bit atomic where the far-pixel count of a source-tile row allows
@@ -158,15 +155,10 @@ def _problem(N, H, W, K, dtype, cfg: WarpLossConfig) -> Problem:
     if dtype not in _DTYPES:
         raise VlgError(f"unsupported activation dtype {dtype}; use float32 or bfloat16")
     flags = (_cabi.FLAG_NO_FAR_PATH if cfg.assume_near else 0) | (0 if cfg.use_tma else _cabi.FLAG_NO_TMA)
-    if cfg.tile_kernels:
-        flags |= _cabi.FLAG_TILE_RGB | _cabi.FLAG_TILE_LAYOUT
     if not cfg.pass2_records:
         flags |= _cabi.FLAG_PASS2_COORDS
     if not cfg.far_packed:
         flags |= _cabi.FLAG_FAR_WIDE
-    if cfg.layout_kernel not in ("tile2", "tile"):
-        raise VlgError(f"layout_kernel must be 'tile2' or 'tile', not {cfg.layout_kernel!r}")
-    flags |= {"tile2": 0, "tile": _cabi.FLAG_TILE_LAYOUT}[cfg.layout_kernel]
     return Problem(N=N, H=H, W=W, K=K, dtype=_DTYPES[dtype], padding=_PADDING[cfg.padding_mode],
                    coord_mode=_cabi.COORD_GRID if cfg.coords_are_grid else _cabi.COORD_FLOW, flags=flags,
                    ignore_index=cfg.ignore_index, w_l1=cfg.w_l1, w_gd=cfg.w_gd, w_ssim=cfg.w_ssim,
