@@ -152,6 +152,21 @@ int vlg_warp_fwd_labels(const vlg_problem_t *prob, const void *src_rgb, const in
 int vlg_colorize(const vlg_problem_t *prob, const void *layout, const int64_t *label,
                  const uint8_t *lut_rgb, void *out_rgb, int64_t *out_label, void *stream);
 
+/* Confusion matrix of predicted layouts against target labels (validation / rollout accuracy; the reference only
+ * dumps torch.argmax(seg, 1), src/trainer.py:342,467).  Rows = target class, columns = predicted class:
+ *   counts[t*K + p] += #{pixels with tgt_label == t and prediction == p}          t, p in [0, K)
+ *   counts[K*K]     += #{pixels skipped because tgt_label or pred_label lies outside [0, K)}
+ * Counts are ADDED (the caller zeroes them once), so batches and rollout steps accumulate without a host sync.
+ *   prediction : pred_label [N,H,W] i64  XOR  argmax_k of `layout` (first max on ties, values as stored -- the
+ *                argmax of vlg_colorize / vlg_warp_fwd)
+ *   layout     : [N,H,W,K] (layout_is_nchw == 0, 16-byte aligned) or [N,K,H,W] contiguous (!= 0), of prob->dtype
+ *   pixels whose tgt_label == prob->ignore_index are not counted anywhere
+ *   counts     : K*K + 1 uint64 on the device
+ * Integer sums: the result is bitwise reproducible whatever the launch configuration.  padding, coord_mode,
+ * weights and flags are ignored. */
+int vlg_confusion(const vlg_problem_t *prob, const void *layout, int32_t layout_is_nchw, const int64_t *pred_label,
+                  const int64_t *tgt_label, uint64_t *counts, void *stream);
+
 /* One-hot layout encoding (src/models/net_utils.py:14-24 transform_seg_one_hot:
  * torch.eye(K)[seg.long()].permute(0,3,1,2)): label [N,H,W] as int64 XOR float32 class ids (the dataset
  * hands float maps, src/folder.py:97-99; values are truncated like .long()) -> layout [N,H,W,K] of the

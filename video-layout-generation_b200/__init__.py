@@ -9,7 +9,8 @@ from ._cabi import VlgError, launch_count  # noqa: F401
 from .graphs import CapturedStep  # noqa: F401
 from .losses import (CombinedLoss, CrossEntropyLoss, GradientLoss, L1Loss, PixelLosses,  # noqa: F401
                      SsimLoss, WarpLoss)
-from .ops import (CITYSCAPES_PALETTE, WarpLossConfig, colorize, empty_nhwc, ingest, one_hot_layout, pixel_losses, prepare_frames,  # noqa: F401
-                  rollout, to_nhwc, warp, warp_labels, warp_loss, warp_loss_labels)
+from .metrics import IoUResult, LayoutIoU  # noqa: F401
+from .ops import (CITYSCAPES_PALETTE, WarpLossConfig, colorize, confusion_matrix, empty_nhwc, ingest, one_hot_layout,  # noqa: F401
+                  pixel_losses, prepare_frames, rollout, to_nhwc, warp, warp_labels, warp_loss, warp_loss_labels)
 
 __version__ = "2.0"

@@ -22,7 +22,8 @@ LOSS_L1, LOSS_GD, LOSS_SSIM, LOSS_CE, LOSS_TV, LOSS_TOTAL, LOSS_NVALID, LOSS_MAX
 ABI_VERSION = 200
 
 EXPORTS = [
-    "vlg_version", "vlg_last_error", "vlg_workspace_bytes", "vlg_warp_fwd", "vlg_warp_fwd_labels", "vlg_colorize", "vlg_one_hot",
+    "vlg_version", "vlg_last_error", "vlg_workspace_bytes", "vlg_warp_fwd", "vlg_warp_fwd_labels", "vlg_colorize", "vlg_confusion",
+    "vlg_one_hot",
     "vlg_frame_affine", "vlg_ingest", "vlg_warp_loss_labels_fwd_bwd",
     "vlg_warp_loss_bwd_out", "vlg_warp_loss_pass1",
     "vlg_warp_bwd_src", "vlg_reduce_partials", "vlg_warp_loss_fwd_bwd", "vlg_pixel_loss_fwd_bwd",
@@ -98,6 +99,8 @@ def load(build_if_missing: bool = True):
     lib.vlg_warp_fwd_labels.argtypes = [P, vp, i64p, f32p, vp, i64p, vp]
     lib.vlg_colorize.argtypes = [P, vp, i64p, vp, vp, i64p, vp]
     lib.vlg_colorize.restype = C.c_int
+    lib.vlg_confusion.argtypes = [P, vp, C.c_int32, i64p, i64p, vp, vp]
+    lib.vlg_confusion.restype = C.c_int
     lib.vlg_one_hot.argtypes = [P, i64p, f32p, vp, vp, vp]
     lib.vlg_one_hot.restype = C.c_int
     lib.vlg_frame_affine.argtypes = [P, f32p, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int32, C.c_int32, vp, i64p, i64p, vp]

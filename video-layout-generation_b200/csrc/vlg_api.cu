@@ -14,6 +14,7 @@
 #include "vlg_frames.cuh"
 #include "vlg_ingest.cuh"
 #include "vlg_labels.cuh"
+#include "vlg_metrics.cuh"
 
 using namespace vlg;
 
@@ -364,12 +365,7 @@ __global__ void __launch_bounds__(256) colorize_kernel(int64_t P, const T *__res
     if (layout) {
         float z[K];
         load_px<T, K>(layout + i * K, z);
-        float m = z[0];
-        int best = 0;
-#pragma unroll
-        for (int k = 1; k < K; ++k)
-            if (z[k] > m) { m = z[k]; best = k; }   // first maximal index
-        l = best;
+        l = first_max_index<K>(z);
         if (out_label) out_label[i] = l;
     } else {
         l = __ldg(label + i);
@@ -481,14 +477,9 @@ __global__ void __launch_bounds__(256) warp_fwd_kernel(CoordCfg cc, int64_t P, i
         }
         if (out_argmax && live) {
             // argmax is taken on the values as STORED (rounded to T), like torch.argmax on the output
-            float m = to_f<T>(from_f<T>(z[0]));
-            int best = 0;
 #pragma unroll
-            for (int k = 1; k < K; ++k) {
-                const float v = to_f<T>(from_f<T>(z[k]));
-                if (v > m) { m = v; best = k; }
-            }
-            out_argmax[i] = best;
+            for (int k = 0; k < K; ++k) z[k] = to_f<T>(from_f<T>(z[k]));
+            out_argmax[i] = first_max_index<K>(z);
         }
     }
 }
@@ -947,6 +938,37 @@ static int launch_colorize(int64_t P, const void *layout, const int64_t *label, 
     return check_launch("colorize_kernel");
 }
 
+// Persistent launch of the confusion-matrix kernel.  Every CTA flushes up to K*K+1 bins with global atomics once, so the
+// grid is one wave of at most kConfMaxCtasPerSm CTAs per SM (4 x 256 threads keep enough 16-byte loads in flight to
+// stream HBM), and no larger than gives every thread kConfMinPxPerThread pixels.
+constexpr int kConfMaxCtasPerSm = 4, kConfMinPxPerThread = 16;
+template <typename T, int K, int MODE>
+static int launch_confusion(const ConfParams &cp, cudaStream_t st) {
+    static PerDevice resident;   // per instantiation
+    int dev = 0;
+    if (int rc = current_device(&dev)) return rc;
+    int ctas = resident.get(dev);
+    if (!ctas) {
+        int per_sm = 0;
+        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, confusion_kernel<T, K, MODE>, kConfThreads, 0);
+        if (e != cudaSuccess || per_sm < 1) return fail(VLG_ERR_CUDA, "confusion_kernel occupancy query: %s", cudaGetErrorString(e));
+        ctas = sm_count() * (per_sm < kConfMaxCtasPerSm ? per_sm : kConfMaxCtasPerSm);
+        resident.set(dev, ctas);
+    }
+    const int64_t by_work = (cp.P + (int64_t)kConfThreads * kConfMinPxPerThread - 1) / ((int64_t)kConfThreads * kConfMinPxPerThread);
+    const int64_t blocks = by_work < ctas ? by_work : ctas;
+    confusion_kernel<T, K, MODE><<<(unsigned)blocks, kConfThreads, 0, st>>>(cp);
+    return check_launch("confusion_kernel");
+}
+
+template <int K>
+static int dispatch_confusion(int dtype, bool layout, bool nchw, const ConfParams &cp, cudaStream_t st) {
+    if (!layout) return launch_confusion<float, K, kConfLabels>(cp, st);   // labels: the problem's dtype plays no part
+    if (dtype == VLG_F32)
+        return nchw ? launch_confusion<float, K, kConfNchw>(cp, st) : launch_confusion<float, K, kConfNhwc>(cp, st);
+    return nchw ? launch_confusion<__nv_bfloat16, K, kConfNchw>(cp, st) : launch_confusion<__nv_bfloat16, K, kConfNhwc>(cp, st);
+}
+
 template <typename T>
 static int launch_frame_affine(const vlg_problem_t *prob, const FrameAffine &fa, const float *in, bool nchw, int flip, void *out, cudaStream_t st) {
     const int64_t P = prob->N * prob->H * prob->W;
@@ -1078,6 +1100,30 @@ int vlg_colorize(const vlg_problem_t *prob, const void *layout, const int64_t *l
     if (prob->K == k)                                                                                     \
         return prob->dtype == VLG_F32 ? launch_colorize<float, k>(P, layout, label, lut_rgb, out_rgb, out_label, st) \
                                       : launch_colorize<__nv_bfloat16, k>(P, layout, label, lut_rgb, out_rgb, out_label, st);
+    VLG_FOR_EACH_K(X)
+#undef X
+    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+}
+
+int vlg_confusion(const vlg_problem_t *prob, const void *layout, int32_t layout_is_nchw, const int64_t *pred_label,
+                  const int64_t *tgt_label, uint64_t *counts, void *stream) {
+    int rc = check_problem(prob);
+    if (rc) return rc;
+    if ((layout == nullptr) == (pred_label == nullptr)) return fail(VLG_ERR_ARG, "give exactly one of layout / pred_label");
+    if (!tgt_label || !counts) return fail(VLG_ERR_ARG, "tgt_label and counts are required");
+    if (layout && !layout_is_nchw && ((uintptr_t)layout & 15)) return fail(VLG_ERR_ARG, "an NHWC layout must be 16-byte aligned");
+    ConfParams cp{};
+    cp.layout = layout;
+    cp.pred = pred_label;
+    cp.tgt = tgt_label;
+    cp.counts = reinterpret_cast<unsigned long long *>(counts);
+    cp.P = prob->N * prob->H * prob->W;
+    cp.ignore_index = prob->ignore_index;
+    cp.HW = (unsigned)(prob->H * prob->W);
+    cp.vec = (((uintptr_t)pred_label | (uintptr_t)tgt_label) & 15) == 0;
+    cudaStream_t st = (cudaStream_t)stream;
+#define X(k) \
+    if (prob->K == k) return dispatch_confusion<k>(prob->dtype, layout != nullptr, layout_is_nchw != 0, cp, st);
     VLG_FOR_EACH_K(X)
 #undef X
     return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");

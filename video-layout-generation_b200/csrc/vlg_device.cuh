@@ -233,6 +233,18 @@ __device__ __forceinline__ void load_px(const T *__restrict__ p, float (&v)[C]) 
     }
 }
 
+// argmax over the K channels of one pixel as torch.argmax takes it (src/trainer.py:342,467): the first maximal index,
+// strict `>` in channel order.  `z` holds the values as stored in the layout's dtype.
+template <int K>
+__device__ __forceinline__ int first_max_index(const float (&z)[K]) {
+    float m = z[0];
+    int best = 0;
+#pragma unroll
+    for (int k = 1; k < K; ++k)
+        if (z[k] > m) { m = z[k]; best = k; }
+    return best;
+}
+
 template <typename T, int C>
 __device__ __forceinline__ void store_px(T *__restrict__ p, const float (&v)[C]) {
     constexpr int VB = vec_bytes(C * (int)sizeof(T));

@@ -298,6 +298,60 @@ def colorize(seg: torch.Tensor, n_classes: int = 20, argmax: bool = False, palet
 
 
 @torch.no_grad()
+def _confusion_into(counts: torch.Tensor, pred: torch.Tensor, target: torch.Tensor, n_classes: int = 20, *,
+                   ignore_index: int = -100):
+    """Adds the confusion counts of (pred, target) into `counts`, one vlg_confusion launch, no synchronisation and no
+    allocation when the inputs need no copy.  `counts` is int64 [K*K + 1] on the device, contiguous: row-major
+    [target, prediction] bins, then the pixels skipped for a label outside [0, K).  `pred` is int64 [N,H,W] class ids or
+    [N,K,H,W] fp32 / bf16 scores (argmax taken on the device; channels_last and plain-contiguous are read as they are,
+    any other stride pattern gets one copy); `target` is int64 [N,H,W]; pixels whose target is `ignore_index` count
+    nowhere."""
+    lib = _cabi.load()
+    dev = _require_cuda(counts, pred, target)
+    K = n_classes
+    if target.dim() != 3:
+        raise VlgError(f"target must be int64 [N,H,W], got shape {tuple(target.shape)}")
+    N, H, W = target.shape
+    _expect(target, (N, H, W), "target", torch.int64)
+    _expect(counts, (K * K + 1,), "counts", torch.int64)
+    if not counts.is_contiguous():
+        raise VlgError("counts must be contiguous")
+    lay = lab = None
+    nchw = 0
+    if pred.dtype == torch.int64:
+        _expect(pred, (N, H, W), "pred (class ids)")
+        lab, dt = pred.contiguous(), torch.float32
+    else:
+        _expect(pred, (N, K, H, W), "pred (scores)")
+        dt = pred.dtype
+        if all(pred.shape[d] == 1 or pred.stride(d) == _nhwc_strides(pred.shape)[d] for d in range(4)):
+            lay = to_nhwc(pred)
+        else:
+            lay, nchw = pred.contiguous(), 1
+    prob = _problem(N, H, W, K, dt, WarpLossConfig(ignore_index=ignore_index))
+    tgt = target.contiguous()
+    with _on(dev):
+        check(lib.vlg_confusion(C.byref(prob), _ptr(lay), nchw, _ptr(lab), _ptr(tgt), _ptr(counts), _stream()))
+
+
+@torch.no_grad()
+def confusion_matrix(pred: torch.Tensor, target: torch.Tensor, n_classes: int = 20, *, ignore_index: int = -100,
+                     debug: bool = False) -> torch.Tensor:
+    """Confusion matrix of a predicted layout against the target labels: int64 [K, K] on the device, rows = target class,
+    columns = predicted class.  `pred` is int64 [N,H,W] class ids or [N,K,H,W] fp32 / bf16 scores, whose argmax (first
+    maximal index, as `torch.argmax(seg, 1)` at src/trainer.py:342) is taken on the device; `target` is int64 [N,H,W].
+    Pixels whose target is `ignore_index` count nowhere; pixels with a target or prediction outside [0, K) count nowhere
+    either -- `debug=True` reads their number (synchronises) and raises if it is not 0."""
+    counts = torch.zeros(n_classes * n_classes + 1, dtype=torch.int64, device=target.device)
+    _confusion_into(counts, pred, target, n_classes, ignore_index=ignore_index)
+    if debug:
+        skipped = int(counts[-1])
+        if skipped:
+            raise VlgError(f"{skipped} pixels have a target or predicted label outside [0, {n_classes}) (and not ignore_index)")
+    return counts[:-1].view(n_classes, n_classes)
+
+
+@torch.no_grad()
 def one_hot_layout(seg: torch.Tensor, n_classes: int = 20, dtype: torch.dtype = torch.float32) -> torch.Tensor:
     """`transform_seg_one_hot` (src/models/net_utils.py:14-24): class-id map -> one-hot layout.
 

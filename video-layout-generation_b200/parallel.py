@@ -65,6 +65,16 @@ def sync_loss_vector(vec: torch.Tensor, convention: str = "global",
     return out
 
 
+def sync_counts(counts: torch.Tensor, group: Optional[dist.ProcessGroup] = None) -> torch.Tensor:
+    """ONE all-reduce (SUM) of int64 counts, e.g. the confusion counts of `metrics.LayoutIoU`: integer sums, so the
+    result equals the single-process counts bit for bit whatever the sharding.  Identity without a process group."""
+    if not (dist.is_available() and dist.is_initialized()):
+        return counts
+    out = counts.clone()
+    dist.all_reduce(out, op=dist.ReduceOp.SUM, group=group)
+    return out
+
+
 def sync_max_disp(vec: torch.Tensor, group: Optional[dist.ProcessGroup] = None) -> torch.Tensor:
     m = vec[SLOT_MAXDISP].clone()
     if dist.is_available() and dist.is_initialized():
