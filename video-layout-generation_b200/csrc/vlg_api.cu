@@ -6,6 +6,7 @@
 #include <cstddef>
 #include <cstdio>
 #include <cstring>
+#include <type_traits>
 
 #include "vlg_pass1.cuh"
 #include "vlg_pass2.cuh"
@@ -104,12 +105,41 @@ static int ensure_smem(PerDevice &done, Kern kern, size_t smem, const char *what
     done.set(dev, 1);
     return VLG_OK;
 }
+// *ctas = CTAs of `kern` (`threads` threads, `smem` bytes of dynamic shared memory) resident at once on the current
+// device, at most `max_per_sm` per SM: one wave of a persistent grid.  Queried once per device into `cache`, which the
+// caller keeps per instantiation.
+template <typename Kern>
+static int resident_ctas(PerDevice &cache, Kern kern, int threads, size_t smem, int max_per_sm, const char *what, int *ctas) {
+    int dev = 0;
+    if (int rc = current_device(&dev)) return rc;
+    *ctas = cache.get(dev);
+    if (*ctas) return VLG_OK;
+    int per_sm = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem);
+    if (e != cudaSuccess || per_sm < 1) return fail(VLG_ERR_CUDA, "%s occupancy query: %s", what, cudaGetErrorString(e));
+    *ctas = sm_count() * (per_sm < max_per_sm ? per_sm : max_per_sm);
+    cache.set(dev, *ctas);
+    return VLG_OK;
+}
 
-static bool k_supported(int64_t K) {
-#define X(k) if (K == k) return true;
+// Calls f(std::integral_constant<int, K>{}) for a K compiled in, fails for any other.
+template <typename F>
+static int with_k(int64_t K, F &&f) {
+#define X(k) if (K == k) return f(std::integral_constant<int, k>{});
     VLG_FOR_EACH_K(X)
 #undef X
-    return false;
+    return fail(VLG_ERR_UNSUPPORTED, "K=%lld not compiled in (see VLG_FOR_EACH_K)", (long long)K);
+}
+// Calls f(type_tag<T>{}) with the element type of a checked dtype.
+template <typename T> struct type_tag { using type = T; };
+template <typename F>
+static int with_type(int dtype, F &&f) {
+    return dtype == VLG_F32 ? f(type_tag<float>{}) : f(type_tag<__nv_bfloat16>{});
+}
+// Calls f(type_tag<T>{}, std::integral_constant<int, K>{}) for the problem's dtype and K.
+template <typename F>
+static int with_type_k(const vlg_problem_t *p, F &&f) {
+    return with_k(p->K, [&](auto k) { return with_type(p->dtype, [&](auto t) { return f(t, k); }); });
 }
 
 static int check_problem(const vlg_problem_t *p) {
@@ -123,7 +153,7 @@ static int check_problem(const vlg_problem_t *p) {
     if (p->N * p->H * p->W >= (1ll << 31)) return fail(VLG_ERR_UNSUPPORTED, "N*H*W must be < 2^31");
     if (p->N > 65535 || (p->H + 7) / 8 > 65535) return fail(VLG_ERR_UNSUPPORTED, "N and H/8 must fit a CUDA grid dimension (65535)");
     if (p->H > 65000 || p->W > 65000) return fail(VLG_ERR_UNSUPPORTED, "H and W must be <= 65000 (16-bit tap cells in the far-pixel queue)");
-    if (!k_supported(p->K)) return fail(VLG_ERR_UNSUPPORTED, "K=%lld not compiled in (see VLG_FOR_EACH_K)", (long long)p->K);
+    if (int rc = with_k(p->K, [](auto) { return VLG_OK; })) return rc;
     if (p->dtype != VLG_F32 && p->dtype != VLG_BF16) return fail(VLG_ERR_ARG, "bad dtype %d", p->dtype);
     if (p->padding != VLG_PAD_ZEROS && p->padding != VLG_PAD_BORDER) return fail(VLG_ERR_ARG, "bad padding %d", p->padding);
     if (p->coord_mode != VLG_COORD_FLOW && p->coord_mode != VLG_COORD_GRID) return fail(VLG_ERR_ARG, "bad coord_mode %d", p->coord_mode);
@@ -137,36 +167,49 @@ static int check_problem(const vlg_problem_t *p) {
     return VLG_OK;
 }
 
-static WsLayout ws_layout(const vlg_problem_t *p, int with_src_grad) {
+// The workspace of a problem: its size, and its arrays for a workspace at `base` (all NULL when `base` is).
+static WsLayout ws_layout(const vlg_problem_t *p, int with_src_grad, void *base = nullptr) {
     WsLayout L{};
     const size_t P = (size_t)p->N * p->H * p->W;
-    L.n_blocks = p->N * tiles_x(p->W) * tiles_y(p->H);
+    const size_t n_blocks = (size_t)(p->N * tiles_x(p->W) * tiles_y(p->H));
     size_t off = 0;
-    L.header = off; off = align_up(off + sizeof(WsHeader), 256);
+    auto take = [&](auto *&array, size_t count) {   // `count` elements, 256-byte aligned
+        array = base ? reinterpret_cast<std::remove_reference_t<decltype(array)>>((char *)base + off) : nullptr;
+        off = align_up(off + count * sizeof(*array), 256);
+    };
     // header, per-tile far flags, per-tile displacement maxima and the far-pixel counts per tile row are contiguous: one memset
     // resets them all
-    L.tile_flags = off; off = align_up(off + (size_t)L.n_blocks * sizeof(uint32_t), 256);
-    L.tile_disp = off; off = align_up(off + (size_t)L.n_blocks * sizeof(float), 256);
-    L.seg_cnt = off; off = align_up(off + (size_t)L.n_blocks * kTH * sizeof(uint32_t), 256);   // far pixels per SOURCE tile row
-    L.partials = off; off = align_up(off + (size_t)L.n_blocks * kPartialSlots * sizeof(float), 256);
-    L.partials_rgb = off; off = align_up(off + (size_t)kRgbMaxWarps * kRgbSlots * sizeof(float), 256);
-    L.partials_lay = off; off = align_up(off + (size_t)kLayMaxWarps * 4 * sizeof(float), 256);
-    L.flagged = off; off = align_up(off + (size_t)L.n_blocks * sizeof(int), 256);
-    L.dout_rgb = L.dout_lay = L.far_acc = L.far_list = L.rec_code = L.rec_frac = 0;
+    take(L.hdr, 1);
+    take(L.tile_flags, n_blocks);
+    take(L.tile_disp, n_blocks);
+    take(L.seg_cnt, n_blocks * kTH);   // far pixels per SOURCE tile row
+    L.zero_bytes = off;
+    take(L.partials, n_blocks * kPartialSlots);
+    take(L.partials_rgb, (size_t)kRgbMaxWarps * kRgbSlots);
+    take(L.partials_lay, (size_t)kLayMaxWarps * 4);
+    take(L.flagged, n_blocks);
     L.pitch = (int64_t)align_up((size_t)p->W, 4);
     if (with_src_grad) {
         const size_t Pp = (size_t)p->N * p->H * (size_t)L.pitch;   // pitched rows: TMA-describable (16-byte row starts)
-        L.dout_rgb = off; off = align_up(off + Pp * 3 * sizeof(float), 256);
-        L.dout_lay = off; off = align_up(off + P * p->K * sizeof(float), 256);
-        L.rec_code = off; off = align_up(off + Pp * sizeof(uint32_t), 256);
-        L.rec_frac = off; off = align_up(off + Pp * sizeof(float2), 256);
+        take(L.dout_rgb, Pp * 3);
+        take(L.dout_lay, P * p->K);
+        take(L.rec_code, Pp);
+        take(L.rec_frac, Pp);
         if (!(p->flags & VLG_FLAG_NO_FAR_PATH)) {
-            L.far_acc = off; off = align_up(off + P * (3 + p->K) * sizeof(long long), 256);
-            L.far_list = off; off = align_up(off + P * sizeof(int4), 256);
+            take(L.far_acc, P * (3 + p->K));
+            take(L.far_list, P);
         }
     }
+    if (p->flags & VLG_FLAG_FAR_WIDE) L.seg_cnt = nullptr;   // without per-row counts pass 2 packs no row
     L.total = off;
     return L;
+}
+
+// The workspace of a checked problem at `workspace`, which must hold at least its total.
+static int workspace_at(const vlg_problem_t *p, int with_src_grad, void *workspace, size_t workspace_bytes, WsLayout *L) {
+    *L = ws_layout(p, with_src_grad, workspace);
+    if (!workspace || workspace_bytes < L->total) return fail(VLG_ERR_WORKSPACE, "workspace too small: need %zu bytes", L->total);
+    return VLG_OK;
 }
 
 static CoordCfg make_cc(const vlg_problem_t *p) {
@@ -258,14 +301,14 @@ static TermCoeffs make_terms(const vlg_problem_t *prob, bool warp) {
     return tc;
 }
 
-static ReduceParams make_reduce_params(const vlg_problem_t *prob, const TermCoeffs &tc, const WsLayout &L, char *ws, float *loss_out) {
+static ReduceParams make_reduce_params(const vlg_problem_t *prob, const TermCoeffs &tc, const WsLayout &L, float *loss_out) {
     const double Ng = (double)(prob->global_N ? prob->global_N : prob->N);
     const double H = (double)prob->H, W = (double)prob->W;
     ReduceParams rp{};
-    rp.partials = (const float *)(ws + L.partials);
-    rp.partials_rgb = (const float *)(ws + L.partials_rgb);
-    rp.partials_lay = (const float *)(ws + L.partials_lay);
-    rp.hdr = (const WsHeader *)(ws + L.header);
+    rp.partials = L.partials;
+    rp.partials_rgb = L.partials_rgb;
+    rp.partials_lay = L.partials_lay;
+    rp.hdr = L.hdr;
     rp.inv_numel_rgb = 1.0 / (Ng * 3 * H * W);
     rp.inv_ssim = (prob->H > 2 && prob->W > 2) ? 1.0 / (Ng * (H - 2) * (W - 2)) : 0.0;
     rp.inv_tvh = 1.0 / (Ng * (H - 1) * W * 2);
@@ -426,14 +469,6 @@ __global__ void __launch_bounds__(256) one_hot_kernel(int64_t P, const int64_t *
     }
 }
 
-template <typename T, int K>
-static int launch_one_hot(int64_t P, const int64_t *lab_i, const float *lab_f, void *out, void *workspace, cudaStream_t st) {
-    constexpr int EPC = 16 / (int)sizeof(T);
-    const int64_t n = (K % EPC) == 0 ? ((P + 31) / 32) * 32 : P;     // a warp per 32 pixels / a thread per pixel
-    one_hot_kernel<T, K><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P, lab_i, lab_f, (T *)out, (WsHeader *)workspace);
-    return check_launch("one_hot_kernel");
-}
-
 // forward-only warp (validation / rollout): one thread per output pixel.  A CTA owns 256 CONSECUTIVE pixels, i.e.
 // 256 * K contiguous elements of the warped layout: with BULK they are staged in shared memory and every warp
 // sends its 32 pixels as one bulk shared->global copy -- a thread-per-pixel store of 80-byte pixels costs 20 L1
@@ -502,25 +537,31 @@ static EncodeTiledFn tensor_map_encoder() {
     return fn;
 }
 
+// Tiled tensor map of a `rank`-D array at `base` (global dims innermost first, the rank-1 byte strides of the outer dims,
+// the box): unit element strides, no interleave, swizzle or out-of-bounds fill.  False when the driver has no encoder or
+// refuses the description.
+static bool encode_map(CUtensorMap *map, CUtensorMapDataType dt, int rank, const void *base, const cuuint64_t *gdim,
+                       const cuuint64_t *gstr, const cuuint32_t *box) {
+    memset(map, 0, sizeof(*map));
+    EncodeTiledFn enc = tensor_map_encoder();
+    if (!enc) return false;
+    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
+    return enc(map, dt, (cuuint32_t)rank, const_cast<void *>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 // Tensor map of an NHWC layout [N][H][W][K] with a box_w x box_h x K box.  Returns false when TMA cannot be used
 // (bf16 K=20 rows are not 16-byte multiples, odd K, ...).
 static bool make_layout_map(const vlg_problem_t *prob, const void *src_layout, CUtensorMap *map, int box_w, int box_h,
                             bool fp32_storage = false) {
-    memset(map, 0, sizeof(*map));
     const size_t es = 4;
     if ((prob->dtype != VLG_F32 && !fp32_storage) || (prob->K * es) % 16 != 0 || prob->K > 256) return false;
     if (((uintptr_t)src_layout) % 16 != 0) return false;
-    EncodeTiledFn enc = tensor_map_encoder();
-    if (!enc) return false;
     const cuuint64_t gdim[4] = {(cuuint64_t)prob->K, (cuuint64_t)prob->W, (cuuint64_t)prob->H, (cuuint64_t)prob->N};
     const cuuint64_t gstr[3] = {(cuuint64_t)prob->K * es, (cuuint64_t)prob->W * prob->K * es,
                                 (cuuint64_t)prob->H * prob->W * prob->K * es};
     const cuuint32_t box[4] = {(cuuint32_t)prob->K, (cuuint32_t)box_w, (cuuint32_t)box_h, 1u};
-    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
-    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void *>(src_layout), gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS;
+    return encode_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, src_layout, gdim, gstr, box);
 }
 
 // Tensor map of an NHWC layout for the persistent tile kernel.  Pixels whose byte size is a multiple of 16
@@ -529,22 +570,15 @@ static bool make_layout_map(const vlg_problem_t *prob, const void *src_layout, C
 static bool make_window_map(const vlg_problem_t *prob, const void *src_layout, CUtensorMap *map, int box_w, int box_h, bool *px8) {
     *px8 = false;
     if (prob->dtype == VLG_F32) return make_layout_map(prob, src_layout, map, box_w, box_h);
-    memset(map, 0, sizeof(*map));
     const size_t pxb = (size_t)prob->K * 2;
     if (pxb % 8 != 0 || ((size_t)prob->W * pxb) % 16 != 0 || ((uintptr_t)src_layout) % 16 != 0) return false;
     const size_t upp = pxb / 8;   // 8-byte units per pixel
     if ((size_t)box_w * upp > 256) return false;
-    EncodeTiledFn enc = tensor_map_encoder();
-    if (!enc) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)prob->W * upp, (cuuint64_t)prob->H, (cuuint64_t)prob->N};
     const cuuint64_t gstr[2] = {(cuuint64_t)prob->W * pxb, (cuuint64_t)prob->H * prob->W * pxb};
     const cuuint32_t box[3] = {(cuuint32_t)(box_w * upp), (cuuint32_t)box_h, 1u};
-    const cuuint32_t estr[3] = {1u, 1u, 1u};
-    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, const_cast<void *>(src_layout), gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    *px8 = r == CUDA_SUCCESS;
-    return r == CUDA_SUCCESS;
+    *px8 = encode_map(map, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, src_layout, gdim, gstr, box);
+    return *px8;
 }
 
 // Pass 2 gathers from the tap records pass 1 wrote (pass2_rec_kernel: all staging by TMA) when the d_out
@@ -558,16 +592,11 @@ static bool pass2_from_records(const vlg_problem_t *prob) {
 // window of kQW2 x kQH pixels.  The tensor's extent along x is W (not the pitch): the padding columns of a row are
 // never written by pass 1, so they must arrive as the TMA's out-of-bounds zeros like every other cell outside the image.
 static bool make_pitched_map(const vlg_problem_t *prob, const void *base, int64_t pitch, int epp, CUtensorMapDataType dt, CUtensorMap *map) {
-    memset(map, 0, sizeof(*map));
     if (((uintptr_t)base) % 16 != 0 || (pitch * epp * 4) % 16 != 0) return false;
-    EncodeTiledFn enc = tensor_map_encoder();
-    if (!enc) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)(prob->W * epp), (cuuint64_t)prob->H, (cuuint64_t)prob->N};
     const cuuint64_t gstr[2] = {(cuuint64_t)(pitch * epp * 4), (cuuint64_t)(prob->H * pitch * epp * 4)};
     const cuuint32_t box[3] = {(cuuint32_t)(kQW2 * epp), (cuuint32_t)kQH, 1u};
-    const cuuint32_t estr[3] = {1u, 1u, 1u};
-    return enc(map, dt, 3, const_cast<void *>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return encode_map(map, dt, 3, base, gdim, gstr, box);
 }
 
 template <typename T, int K>
@@ -582,16 +611,6 @@ static int launch_pass1(bool warp, const Pass1Params &pp, cudaStream_t st) {
     if (warp) pass1_kernel<T, K, true><<<grid, kThreads, smem_warp, st>>>(pp);
     else pass1_kernel<T, K, false><<<grid, kThreads, smem_plain, st>>>(pp);
     return check_launch("pass1_kernel");
-}
-
-static int dispatch_pass1(const vlg_problem_t *prob, bool warp, const Pass1Params &pp, cudaStream_t st) {
-#define X(k)                                                                                                              \
-    if (prob->K == k) {                                                                                                   \
-        return prob->dtype == VLG_F32 ? launch_pass1<float, k>(warp, pp, st) : launch_pass1<__nv_bfloat16, k>(warp, pp, st); \
-    }
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
 }
 
 template <typename T, int K>
@@ -659,16 +678,9 @@ static int launch_fwd(const vlg_problem_t *prob, const void *src_rgb, const void
 template <typename T>
 static int launch_rgb(RgbParams rp, bool grad, cudaStream_t st) {
     static PerDevice resident;   // per instantiation (T); GRAD variants share the register budget
-    int dev = 0;
-    if (int rc = current_device(&dev)) return rc;
-    int warps_resident = resident.get(dev);
-    if (!warps_resident) {
-        int per_sm = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rgb_strip_kernel<T, true, false>, kRgbThreads, 0);
-        if (e != cudaSuccess || per_sm < 1) return fail(VLG_ERR_CUDA, "rgb_strip_kernel occupancy query: %s", cudaGetErrorString(e));
-        warps_resident = sm_count() * per_sm * (kRgbThreads / 32);
-        resident.set(dev, warps_resident);
-    }
+    int ctas = 0;
+    if (int rc = resident_ctas(resident, rgb_strip_kernel<T, true, false>, kRgbThreads, 0, INT_MAX, "rgb_strip_kernel", &ctas)) return rc;
+    const int warps_resident = ctas * (kRgbThreads / 32);
     int64_t warps = warps_resident < kRgbMaxWarps ? warps_resident : kRgbMaxWarps;
     const int64_t min_rows = 12;   // shorter runs are dominated by the 4 warm-up rows of a segment
     if (warps * min_rows > rp.total_rows) warps = (rp.total_rows + min_rows - 1) / min_rows;
@@ -687,18 +699,11 @@ template <typename T, int K, bool PX8>
 static int launch_laytile(const LayParams &lp, const CUtensorMap &map, bool grad, cudaStream_t st) {
     const size_t smem = sizeof(LayTileSmem<T, K>);
     static PerDevice resident, attr_g, attr_n;
-    int dev = 0;
-    if (int rc = current_device(&dev)) return rc;
     if (int rc = ensure_smem(attr_g, lay_tile_kernel<T, K, true, PX8>, smem, "lay_tile")) return rc;
     if (int rc = ensure_smem(attr_n, lay_tile_kernel<T, K, false, PX8>, smem, "lay_tile")) return rc;
-    int ctas_resident = resident.get(dev);
-    if (!ctas_resident) {
-        int per_sm = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lay_tile_kernel<T, K, true, PX8>, kThreads, smem);
-        if (e != cudaSuccess || per_sm < 1) return fail(VLG_ERR_CUDA, "lay_tile_kernel setup: %s", cudaGetErrorString(e));
-        ctas_resident = sm_count() * per_sm;
-        resident.set(dev, ctas_resident);
-    }
+    int ctas_resident = 0;
+    if (int rc = resident_ctas(resident, lay_tile_kernel<T, K, true, PX8>, kThreads, smem, INT_MAX, "lay_tile_kernel", &ctas_resident))
+        return rc;
     const int64_t n_tiles = (int64_t)lp.N * lp.strips * lp.tiles_y;
     int64_t blocks = ctas_resident < kLayMaxWarps ? ctas_resident : kLayMaxWarps;
     if (blocks * 2 > n_tiles) blocks = (n_tiles + 1) / 2;    // at least two tiles per CTA keeps the pipeline meaningful
@@ -708,25 +713,11 @@ static int launch_laytile(const LayParams &lp, const CUtensorMap &map, bool grad
     return check_launch("lay_tile_kernel");
 }
 
-static int dispatch_laytile(const vlg_problem_t *prob, const LayParams &lp, const CUtensorMap &map, bool px8, bool grad, cudaStream_t st) {
-#define X(k)                                                                                                   \
-    if constexpr ((k) % 4 == 0) {                                                                              \
-        if (prob->K == k) {                                                                                    \
-            if (prob->dtype == VLG_F32) return launch_laytile<float, k, false>(lp, map, grad, st);             \
-            if (px8) return launch_laytile<__nv_bfloat16, k, true>(lp, map, grad, st);                         \
-            if constexpr ((k) % 8 == 0) return launch_laytile<__nv_bfloat16, k, false>(lp, map, grad, st);     \
-        }                                                                                                      \
-    }
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "layout tile kernel: K / dtype not compiled in");
-}
-
 // The rgb strip kernel with the gradient scales of `tc`: d(loss)/d(coords) (rgb part, nullable), the d(loss)/d(warped rgb)
 // staging for pass 2 (nullable) and one partial row per warp.
 static int launch_rgb_strips(const vlg_problem_t *prob, const TermCoeffs &tc, const void *src_rgb, const void *tgt_rgb,
                              const float *coords, float *d_coords, float *d_out_rgb, bool need_grad, const WsLayout &L,
-                             char *ws, cudaStream_t st) {
+                             cudaStream_t st) {
     RgbParams rp{};
     rp.cc = make_cc(prob);
     rp.N = (int)prob->N;
@@ -737,9 +728,9 @@ static int launch_rgb_strips(const vlg_problem_t *prob, const TermCoeffs &tc, co
     rp.d_coords = d_coords;
     rp.d_out_rgb = d_out_rgb;
     rp.pitch = (int)L.pitch;
-    rp.partials = (float *)(ws + L.partials_rgb);
-    rp.hdr = (WsHeader *)(ws + L.header);
-    return prob->dtype == VLG_F32 ? launch_rgb<float>(rp, need_grad, st) : launch_rgb<__nv_bfloat16>(rp, need_grad, st);
+    rp.partials = L.partials_rgb;
+    rp.hdr = L.hdr;
+    return with_type(prob->dtype, [&](auto t) { return launch_rgb<typename decltype(t)::type>(rp, need_grad, st); });
 }
 
 // Side stream + fork/join events of the calling thread, one lane per device (created on first use).  Used to run the
@@ -805,11 +796,10 @@ static int count_beside_rgb(const vlg_problem_t *prob, bool count, const int64_t
 static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, const void *src_layout,
                      const float *coords, const void *tgt_rgb, const int64_t *tgt_label, float *d_coords,
                      void *d_out_rgb, void *d_out_lay, bool need_grad, int64_t *out_argmax, float *fused_loss_out,
-                     void *workspace, const WsLayout &L, cudaStream_t st) {
-    char *ws = (char *)workspace;
-    WsHeader *hdr = (WsHeader *)(ws + L.header);
+                     const WsLayout &L, cudaStream_t st) {
+    WsHeader *hdr = L.hdr;
     // header + per-tile far flags + per-tile displacement maxima are contiguous: one memset node resets them
-    cudaError_t e = cudaMemsetAsync(hdr, 0, L.partials - L.header, st);
+    cudaError_t e = cudaMemsetAsync(hdr, 0, L.zero_bytes, st);
     if (e != cudaSuccess) return fail(VLG_ERR_CUDA, "memset header: %s", cudaGetErrorString(e));
     const int64_t P = prob->N * prob->H * prob->W;
     const bool has_lay = src_layout && tgt_label;
@@ -821,7 +811,7 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     int rc = count_beside_rgb(prob, has_lay, tgt_label, hdr, rgb_strips, [&] {
         tl_mark(kTlRgb0, st);
         const int r = launch_rgb_strips(prob, tc, src_rgb, tgt_rgb, coords, need_grad ? d_coords : nullptr,
-                                        need_grad ? (float *)d_out_rgb : nullptr, need_grad, L, ws, st);
+                                        need_grad ? (float *)d_out_rgb : nullptr, need_grad, L, st);
         tl_mark(kTlRgb1, st);
         return r;
     }, st);
@@ -838,17 +828,17 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
     pp.need_grad = need_grad;
     pp.d_coords = d_coords; pp.d_out_rgb = d_out_rgb; pp.d_out_lay = d_out_lay;
     pp.out_argmax = out_argmax;
-    pp.partials = (float *)(ws + L.partials);
-    pp.tile_disp = (float *)(ws + L.tile_disp);
-    pp.tile_flags = (uint32_t *)(ws + L.tile_flags);
-    pp.seg_cnt = (prob->flags & VLG_FLAG_FAR_WIDE) ? nullptr : (uint32_t *)(ws + L.seg_cnt);
-    pp.far_list = (warp && d_out_lay && L.far_list) ? (int4 *)(ws + L.far_list) : nullptr;
-    pp.flagged_list = (int *)(ws + L.flagged);
-    pp.red = make_reduce_params(prob, tc, L, ws, fused_loss_out);
+    pp.partials = L.partials;
+    pp.tile_disp = L.tile_disp;
+    pp.tile_flags = L.tile_flags;
+    pp.seg_cnt = L.seg_cnt;
+    pp.far_list = (warp && d_out_lay) ? L.far_list : nullptr;
+    pp.flagged_list = L.flagged;
+    pp.red = make_reduce_params(prob, tc, L, fused_loss_out);
     pp.hdr = hdr;
     pp.accum_dcoords = rgb_strips ? 1 : 0;
     // tap records for pass 2: written by lay_tile_kernel on its way, by tap_records_kernel after pass1_kernel
-    const bool want_records = warp && need_grad && d_out_lay != nullptr && L.rec_code != 0 && pass2_from_records(prob);
+    const bool want_records = warp && need_grad && d_out_lay != nullptr && L.rec_code && pass2_from_records(prob);
     bool records_done = false;
     bool lay_done = false;
     if (warp && has_lay && prob->K % 4 == 0 && !(prob->flags & VLG_FLAG_NO_TMA)) {
@@ -866,27 +856,39 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
             lp.d_coords = need_grad ? d_coords : nullptr;
             lp.d_out_lay = need_grad ? (float *)d_out_lay : nullptr;
             if (want_records) {
-                lp.rec_code = (uint32_t *)(ws + L.rec_code); lp.rec_frac = (float2 *)(ws + L.rec_frac); lp.pitch = (int)L.pitch;
+                lp.rec_code = L.rec_code; lp.rec_frac = L.rec_frac; lp.pitch = (int)L.pitch;
                 records_done = true;
             }
             lp.out_argmax = out_argmax;
-            lp.partials = (float *)(ws + L.partials_lay);
+            lp.partials = L.partials_lay;
             lp.tile_disp = pp.tile_disp; lp.far_list = pp.far_list; lp.tile_flags = pp.tile_flags; lp.seg_cnt = pp.seg_cnt; lp.flagged_list = pp.flagged_list;
             lp.red = pp.red; lp.hdr = hdr;
             tl_mark(kTlLay0, st);
-            rc = dispatch_laytile(prob, lp, row_map, px8, need_grad, st);
+            // lay_tile_kernel is compiled for K % 4 == 0: fp32, and bf16 in 8-byte units (PX8) or with K % 8 == 0
+            rc = with_type_k(prob, [&](auto t, auto k) {
+                using T = typename decltype(t)::type;
+                constexpr int K = decltype(k)::value;
+                constexpr bool f32 = std::is_same<T, float>::value;
+                if constexpr (K % 4 == 0 && !f32) {
+                    if (px8) return launch_laytile<T, K, true>(lp, row_map, need_grad, st);
+                }
+                if constexpr (K % 4 == 0 && (f32 || K % 8 == 0)) {
+                    if (!px8) return launch_laytile<T, K, false>(lp, row_map, need_grad, st);
+                }
+                return fail(VLG_ERR_UNSUPPORTED, "layout tile kernel: K / dtype not compiled in");
+            });
             tl_mark(kTlLay1, st);
             if (rc) return rc;
             lay_done = true;
         }
     }
     if (!lay_done) {
-        rc = dispatch_pass1(prob, warp, pp, st);
+        rc = with_type_k(prob, [&](auto t, auto k) { return launch_pass1<typename decltype(t)::type, decltype(k)::value>(warp, pp, st); });
         if (rc) return rc;
     }
     if (want_records && !records_done) {
         tap_records_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(pp.cc, P, prob->H * prob->W, (int)L.pitch, (const float2 *)coords,
-                                                                        (uint32_t *)(ws + L.rec_code), (float2 *)(ws + L.rec_frac));
+                                                                        L.rec_code, L.rec_frac);
         rc = check_launch("tap_records_kernel");
     }
     return rc;
@@ -896,19 +898,18 @@ static int run_pass1(const vlg_problem_t *prob, bool warp, const void *src_rgb, 
 // join -> lab_pix_kernel (layout terms from four label taps, TV, sum of d_coords, final reduction).
 static int run_pass1_labels(const vlg_problem_t *prob, const void *src_rgb, const int64_t *src_label, const float *coords,
                             const void *tgt_rgb, const int64_t *tgt_label, float *d_coords, int64_t *out_argmax, float *loss_out,
-                            void *workspace, const WsLayout &L, cudaStream_t st) {
-    char *ws = (char *)workspace;
-    WsHeader *hdr = (WsHeader *)(ws + L.header);
+                            const WsLayout &L, cudaStream_t st) {
+    WsHeader *hdr = L.hdr;
     const int64_t P = prob->N * prob->H * prob->W;
     const bool has_rgb = src_rgb && tgt_rgb;
     if (!(src_label && tgt_label)) return fail(VLG_ERR_UNSUPPORTED, "the label-source op needs src_label / tgt_label (use vlg_pixel_loss_* for rgb-only criteria)");
-    cudaError_t e = cudaMemsetAsync(hdr, 0, L.partials - L.header, st);
+    cudaError_t e = cudaMemsetAsync(hdr, 0, L.zero_bytes, st);
     if (e != cudaSuccess) return fail(VLG_ERR_CUDA, "memset header: %s", cudaGetErrorString(e));
     const bool need_grad = d_coords != nullptr;
     const TermCoeffs tc = make_terms(prob, true);
     // sources are data: no pass 2, no d(loss)/d(warped rgb) staging
     int rc = count_beside_rgb(prob, true, tgt_label, hdr, has_rgb, [&] {
-        return launch_rgb_strips(prob, tc, src_rgb, tgt_rgb, coords, d_coords, nullptr, need_grad, L, ws, st);
+        return launch_rgb_strips(prob, tc, src_rgb, tgt_rgb, coords, d_coords, nullptr, need_grad, L, st);
     }, st);
     if (rc) return rc;
     LabParams lp{};
@@ -918,8 +919,8 @@ static int run_pass1_labels(const vlg_problem_t *prob, const void *src_rgb, cons
     lp.tc = tc;
     lp.accum_dcoords = has_rgb ? 1 : 0;
     lp.d_coords = d_coords; lp.out_argmax = out_argmax;
-    lp.partials = (float *)(ws + L.partials_lay);
-    lp.red = make_reduce_params(prob, tc, L, ws, loss_out);
+    lp.partials = L.partials_lay;
+    lp.red = make_reduce_params(prob, tc, L, loss_out);
     lp.hdr = hdr;
     int64_t blocks = (int64_t)sm_count() * 8;
     const int64_t max_blocks = (P + kLabThreads - 1) / kLabThreads;
@@ -930,14 +931,6 @@ static int run_pass1_labels(const vlg_problem_t *prob, const void *src_rgb, cons
     return check_launch("lab_pix_kernel");
 }
 
-template <typename T, int K>
-static int launch_colorize(int64_t P, const void *layout, const int64_t *label, const uint8_t *lut, void *out_rgb,
-                           int64_t *out_label, cudaStream_t st) {
-    colorize_kernel<T, K><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(P, (const T *)layout, label, lut, (T *)out_rgb,
-                                                                      out_label, nullptr);
-    return check_launch("colorize_kernel");
-}
-
 // Persistent launch of the confusion-matrix kernel.  Every CTA flushes up to K*K+1 bins with global atomics once, so the
 // grid is one wave of at most kConfMaxCtasPerSm CTAs per SM (4 x 256 threads keep enough 16-byte loads in flight to
 // stream HBM), and no larger than gives every thread kConfMinPxPerThread pixels.
@@ -945,28 +938,13 @@ constexpr int kConfMaxCtasPerSm = 4, kConfMinPxPerThread = 16;
 template <typename T, int K, int MODE>
 static int launch_confusion(const ConfParams &cp, cudaStream_t st) {
     static PerDevice resident;   // per instantiation
-    int dev = 0;
-    if (int rc = current_device(&dev)) return rc;
-    int ctas = resident.get(dev);
-    if (!ctas) {
-        int per_sm = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, confusion_kernel<T, K, MODE>, kConfThreads, 0);
-        if (e != cudaSuccess || per_sm < 1) return fail(VLG_ERR_CUDA, "confusion_kernel occupancy query: %s", cudaGetErrorString(e));
-        ctas = sm_count() * (per_sm < kConfMaxCtasPerSm ? per_sm : kConfMaxCtasPerSm);
-        resident.set(dev, ctas);
-    }
+    int ctas = 0;
+    if (int rc = resident_ctas(resident, confusion_kernel<T, K, MODE>, kConfThreads, 0, kConfMaxCtasPerSm, "confusion_kernel", &ctas))
+        return rc;
     const int64_t by_work = (cp.P + (int64_t)kConfThreads * kConfMinPxPerThread - 1) / ((int64_t)kConfThreads * kConfMinPxPerThread);
     const int64_t blocks = by_work < ctas ? by_work : ctas;
     confusion_kernel<T, K, MODE><<<(unsigned)blocks, kConfThreads, 0, st>>>(cp);
     return check_launch("confusion_kernel");
-}
-
-template <int K>
-static int dispatch_confusion(int dtype, bool layout, bool nchw, const ConfParams &cp, cudaStream_t st) {
-    if (!layout) return launch_confusion<float, K, kConfLabels>(cp, st);   // labels: the problem's dtype plays no part
-    if (dtype == VLG_F32)
-        return nchw ? launch_confusion<float, K, kConfNchw>(cp, st) : launch_confusion<float, K, kConfNhwc>(cp, st);
-    return nchw ? launch_confusion<__nv_bfloat16, K, kConfNchw>(cp, st) : launch_confusion<__nv_bfloat16, K, kConfNhwc>(cp, st);
 }
 
 template <typename T>
@@ -1059,14 +1037,10 @@ int vlg_warp_fwd(const vlg_problem_t *prob, const void *src_rgb, const void *src
     if (rc) return rc;
     if (!coords) return fail(VLG_ERR_ARG, "coords is NULL");
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k)                                                                                                   \
-    if (prob->K == k)                                                                                          \
-        return prob->dtype == VLG_F32                                                                          \
-                   ? launch_fwd<float, k>(prob, src_rgb, src_layout, coords, out_rgb, out_layout, out_argmax, dbg_x0y0, st) \
-                   : launch_fwd<__nv_bfloat16, k>(prob, src_rgb, src_layout, coords, out_rgb, out_layout, out_argmax, dbg_x0y0, st);
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+    return with_type_k(prob, [&](auto t, auto k) {
+        return launch_fwd<typename decltype(t)::type, decltype(k)::value>(prob, src_rgb, src_layout, coords, out_rgb, out_layout,
+                                                                          out_argmax, dbg_x0y0, st);
+    });
 }
 
 int vlg_warp_fwd_labels(const vlg_problem_t *prob, const void *src_rgb, const int64_t *src_label, const float *coords,
@@ -1077,15 +1051,12 @@ int vlg_warp_fwd_labels(const vlg_problem_t *prob, const void *src_rgb, const in
     if ((src_label == nullptr) != (out_label == nullptr)) return fail(VLG_ERR_ARG, "src_label and out_label go together");
     const int64_t HW = prob->H * prob->W, P = prob->N * HW;
     cudaStream_t st = (cudaStream_t)stream;
-    const unsigned blocks = (unsigned)((P + 255) / 256);
-    if (prob->dtype == VLG_F32)
-        warp_fwd_labels_kernel<float><<<blocks, 256, 0, st>>>(make_cc(prob), P, HW, (const float *)src_rgb, src_label,
-                                                              (const float2 *)coords, (float *)out_rgb, out_label);
-    else
-        warp_fwd_labels_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(make_cc(prob), P, HW, (const __nv_bfloat16 *)src_rgb,
-                                                                      src_label, (const float2 *)coords,
-                                                                      (__nv_bfloat16 *)out_rgb, out_label);
-    return check_launch("warp_fwd_labels_kernel");
+    return with_type(prob->dtype, [&](auto t) {
+        using T = typename decltype(t)::type;
+        warp_fwd_labels_kernel<T><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(make_cc(prob), P, HW, (const T *)src_rgb, src_label,
+                                                                               (const float2 *)coords, (T *)out_rgb, out_label);
+        return check_launch("warp_fwd_labels_kernel");
+    });
 }
 
 int vlg_colorize(const vlg_problem_t *prob, const void *layout, const int64_t *label, const uint8_t *lut_rgb,
@@ -1096,13 +1067,12 @@ int vlg_colorize(const vlg_problem_t *prob, const void *layout, const int64_t *l
     if (!lut_rgb || !out_rgb) return fail(VLG_ERR_ARG, "lut_rgb and out_rgb are required");
     const int64_t P = prob->N * prob->H * prob->W;
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k)                                                                                              \
-    if (prob->K == k)                                                                                     \
-        return prob->dtype == VLG_F32 ? launch_colorize<float, k>(P, layout, label, lut_rgb, out_rgb, out_label, st) \
-                                      : launch_colorize<__nv_bfloat16, k>(P, layout, label, lut_rgb, out_rgb, out_label, st);
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+    return with_type_k(prob, [&](auto t, auto k) {
+        using T = typename decltype(t)::type;
+        colorize_kernel<T, decltype(k)::value><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(P, (const T *)layout, label, lut_rgb,
+                                                                                         (T *)out_rgb, out_label, nullptr);
+        return check_launch("colorize_kernel");
+    });
 }
 
 int vlg_confusion(const vlg_problem_t *prob, const void *layout, int32_t layout_is_nchw, const int64_t *pred_label,
@@ -1122,11 +1092,14 @@ int vlg_confusion(const vlg_problem_t *prob, const void *layout, int32_t layout_
     cp.HW = (unsigned)(prob->H * prob->W);
     cp.vec = (((uintptr_t)pred_label | (uintptr_t)tgt_label) & 15) == 0;
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k) \
-    if (prob->K == k) return dispatch_confusion<k>(prob->dtype, layout != nullptr, layout_is_nchw != 0, cp, st);
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+    return with_k(prob->K, [&](auto k) {
+        constexpr int K = decltype(k)::value;
+        if (!layout) return launch_confusion<float, K, kConfLabels>(cp, st);   // labels: the problem's dtype plays no part
+        return with_type(prob->dtype, [&](auto t) {
+            using T = typename decltype(t)::type;
+            return layout_is_nchw ? launch_confusion<T, K, kConfNchw>(cp, st) : launch_confusion<T, K, kConfNhwc>(cp, st);
+        });
+    });
 }
 
 int vlg_one_hot(const vlg_problem_t *prob, const int64_t *label_i64, const float *label_f32, void *out_layout,
@@ -1137,29 +1110,26 @@ int vlg_one_hot(const vlg_problem_t *prob, const int64_t *label_i64, const float
     if (!out_layout) return fail(VLG_ERR_ARG, "out_layout is NULL");
     const int64_t P = prob->N * prob->H * prob->W;
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k)                                                                                                  \
-    if (prob->K == k)                                                                                         \
-        return prob->dtype == VLG_F32 ? launch_one_hot<float, k>(P, label_i64, label_f32, out_layout, workspace, st) \
-                                      : launch_one_hot<__nv_bfloat16, k>(P, label_i64, label_f32, out_layout, workspace, st);
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+    return with_type_k(prob, [&](auto t, auto k) {
+        using T = typename decltype(t)::type;
+        constexpr int K = decltype(k)::value, EPC = 16 / (int)sizeof(T);
+        const int64_t n = (K % EPC) == 0 ? ((P + 31) / 32) * 32 : P;     // a warp per 32 pixels / a thread per pixel
+        one_hot_kernel<T, K><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P, label_i64, label_f32, (T *)out_layout, (WsHeader *)workspace);
+        return check_launch("one_hot_kernel");
+    });
 }
 
 static int warp_loss_pass1(const vlg_problem_t *prob, const void *src_rgb, const void *src_layout, const float *coords,
                            const void *tgt_rgb, const int64_t *tgt_label, float *d_coords, int64_t *out_argmax,
                            int with_src_grad, float *fused_loss_out, void *workspace, size_t workspace_bytes,
                            void *stream) {
-    int rc = check_problem(prob);
-    if (rc) return rc;
+    if (int rc = check_problem(prob)) return rc;
     if (!coords) return fail(VLG_ERR_ARG, "coords is NULL");
     if (with_src_grad && !d_coords) return fail(VLG_ERR_ARG, "with_src_grad needs d_coords (gradient pass)");
-    const WsLayout L = ws_layout(prob, with_src_grad);
-    if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small: need %zu bytes", L.total);
-    char *ws = (char *)workspace;
-    return run_pass1(prob, true, src_rgb, src_layout, coords, tgt_rgb, tgt_label, d_coords,
-                     with_src_grad ? ws + L.dout_rgb : nullptr, with_src_grad ? ws + L.dout_lay : nullptr,
-                     d_coords != nullptr, out_argmax, fused_loss_out, workspace, L, (cudaStream_t)stream);
+    WsLayout L;
+    if (int rc = workspace_at(prob, with_src_grad, workspace, workspace_bytes, &L)) return rc;
+    return run_pass1(prob, true, src_rgb, src_layout, coords, tgt_rgb, tgt_label, d_coords, L.dout_rgb, L.dout_lay,
+                     d_coords != nullptr, out_argmax, fused_loss_out, L, (cudaStream_t)stream);
 }
 
 int vlg_warp_loss_bwd_out(const vlg_problem_t *prob, const void *src_rgb, const void *src_layout, const float *coords,
@@ -1178,47 +1148,38 @@ int vlg_warp_loss_pass1(const vlg_problem_t *prob, const void *src_rgb, const vo
 
 int vlg_warp_bwd_src(const vlg_problem_t *prob, const float *coords, void *d_src_rgb, void *d_src_layout,
                      void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = check_problem(prob);
-    if (rc) return rc;
+    if (int rc = check_problem(prob)) return rc;
     if (!coords) return fail(VLG_ERR_ARG, "coords is NULL");
-    const WsLayout L = ws_layout(prob, 1);
-    if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small: need %zu bytes", L.total);
-    char *ws = (char *)workspace;
+    WsLayout L;
+    if (int rc = workspace_at(prob, 1, workspace, workspace_bytes, &L)) return rc;
     Pass2Params pp{};
     pp.cc = make_cc(prob);
     pp.N = (int)prob->N; pp.tiles_x = (int)tiles_x(prob->W); pp.tiles_y = (int)tiles_y(prob->H);
     pp.coords = coords;
-    pp.d_out_rgb = (const float *)(ws + L.dout_rgb);
-    pp.d_out_lay = (const float *)(ws + L.dout_lay);
-    pp.rec_code = (const uint32_t *)(ws + L.rec_code);
-    pp.rec_frac = (const float2 *)(ws + L.rec_frac);
+    pp.d_out_rgb = L.dout_rgb;
+    pp.d_out_lay = L.dout_lay;
+    pp.rec_code = L.rec_code;
+    pp.rec_frac = L.rec_frac;
     pp.pitch = (int)L.pitch;
     pp.d_src_rgb = d_src_rgb; pp.d_src_lay = d_src_layout;
-    pp.far_acc = L.far_acc ? (long long *)(ws + L.far_acc) : nullptr;
-    pp.far_list = L.far_list ? (const int4 *)(ws + L.far_list) : nullptr;
-    pp.tile_flags = (const uint32_t *)(ws + L.tile_flags);
-    pp.seg_cnt = (prob->flags & VLG_FLAG_FAR_WIDE) ? nullptr : (const uint32_t *)(ws + L.seg_cnt);
-    pp.flagged_list = (const int *)(ws + L.flagged);
-    pp.hdr = (WsHeader *)(ws + L.header);
-    pp.tile_disp = (const float *)(ws + L.tile_disp);
+    pp.far_acc = L.far_acc;
+    pp.far_list = L.far_list;
+    pp.tile_flags = L.tile_flags;
+    pp.seg_cnt = L.seg_cnt;
+    pp.flagged_list = L.flagged;
+    pp.hdr = L.hdr;
+    pp.tile_disp = L.tile_disp;
     pp.HW = prob->H * prob->W;
     cudaStream_t st = (cudaStream_t)stream;
-#define X(k)                                                                                                         \
-    if (prob->K == k)                                                                                                \
-        return prob->dtype == VLG_F32 ? launch_pass2<float, k>(pp, prob, st) : launch_pass2<__nv_bfloat16, k>(pp, prob, st);
-    VLG_FOR_EACH_K(X)
-#undef X
-    return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+    return with_type_k(prob, [&](auto t, auto k) { return launch_pass2<typename decltype(t)::type, decltype(k)::value>(pp, prob, st); });
 }
 
 int vlg_reduce_partials(const vlg_problem_t *prob, float *loss_out, void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = check_problem(prob);
-    if (rc) return rc;
+    if (int rc = check_problem(prob)) return rc;
     if (!loss_out) return fail(VLG_ERR_ARG, "loss_out is NULL");
-    const WsLayout L = ws_layout(prob, 0);
-    if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small");
-    char *ws = (char *)workspace;
-    const ReduceParams rp = make_reduce_params(prob, make_terms(prob, true), L, ws, loss_out);
+    WsLayout L;
+    if (int rc = workspace_at(prob, 0, workspace, workspace_bytes, &L)) return rc;
+    const ReduceParams rp = make_reduce_params(prob, make_terms(prob, true), L, loss_out);
     reduce_partials_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(rp);
     return check_launch("reduce_partials_kernel");
 }
@@ -1239,16 +1200,14 @@ int vlg_warp_loss_fwd_bwd(const vlg_problem_t *prob, const void *src_rgb, const 
 int vlg_warp_loss_labels_fwd_bwd(const vlg_problem_t *prob, const void *src_rgb, const int64_t *src_label, const float *coords,
                                  const void *tgt_rgb, const int64_t *tgt_label, float *loss_out, float *d_coords,
                                  int64_t *out_argmax, void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = check_problem(prob);
-    if (rc) return rc;
+    if (int rc = check_problem(prob)) return rc;
     if (!coords) return fail(VLG_ERR_ARG, "coords is NULL");
     if ((src_rgb == nullptr) != (tgt_rgb == nullptr)) return fail(VLG_ERR_ARG, "src_rgb and tgt_rgb go together");
     if ((src_label == nullptr) != (tgt_label == nullptr)) return fail(VLG_ERR_ARG, "src_label and tgt_label go together");
     if (!src_rgb && !src_label) return fail(VLG_ERR_ARG, "nothing to evaluate");
-    const WsLayout L = ws_layout(prob, 0);
-    if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small: need %zu bytes", L.total);
-    return run_pass1_labels(prob, src_rgb, src_label, coords, tgt_rgb, tgt_label, d_coords, out_argmax, loss_out, workspace, L,
-                            (cudaStream_t)stream);
+    WsLayout L;
+    if (int rc = workspace_at(prob, 0, workspace, workspace_bytes, &L)) return rc;
+    return run_pass1_labels(prob, src_rgb, src_label, coords, tgt_rgb, tgt_label, d_coords, out_argmax, loss_out, L, (cudaStream_t)stream);
 }
 
 int vlg_ingest(const vlg_problem_t *prob, const uint8_t *frames_u8, const float *mean3, const float *std3, int32_t flip_w,
@@ -1269,28 +1228,19 @@ int vlg_ingest(const vlg_problem_t *prob, const uint8_t *frames_u8, const float 
         nm.normalize = mean3 != nullptr;
         for (int c = 0; c < 3; ++c) { nm.mean[c] = mean3 ? mean3[c] : 0.f; nm.std[c] = std3 ? std3[c] : 1.f; }
         const bool vec = W % 4 == 0 && ((uintptr_t)frames_u8) % 4 == 0 && ((uintptr_t)out_frames) % 16 == 0;
-        if (vec) {
-            const int64_t groups = P / 4;
-            const unsigned blocks = (unsigned)((groups + 255) / 256);
-            if (prob->dtype == VLG_F32) ingest_frames_vec4_kernel<float><<<blocks, 256, 0, st>>>(nm, groups, W, flip, frames_u8, (float *)out_frames);
-            else ingest_frames_vec4_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(nm, groups, W, flip, frames_u8, (__nv_bfloat16 *)out_frames);
-        } else {
-            const unsigned blocks = (unsigned)((P + 255) / 256);
-            if (prob->dtype == VLG_F32) ingest_frames_px_kernel<float><<<blocks, 256, 0, st>>>(nm, P, W, flip, frames_u8, (float *)out_frames);
-            else ingest_frames_px_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(nm, P, W, flip, frames_u8, (__nv_bfloat16 *)out_frames);
-        }
-        rc = check_launch("ingest_frames_kernel");
+        rc = with_type(prob->dtype, [&](auto t) {
+            using T = typename decltype(t)::type;
+            if (vec) ingest_frames_vec4_kernel<T><<<(unsigned)((P / 4 + 255) / 256), 256, 0, st>>>(nm, P / 4, W, flip, frames_u8, (T *)out_frames);
+            else ingest_frames_px_kernel<T><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(nm, P, W, flip, frames_u8, (T *)out_frames);
+            return check_launch("ingest_frames_kernel");
+        });
         if (rc) return rc;
     }
     if (seg_u8) {
-#define X(k)                                                                                                                       \
-        if (prob->K == k) {                                                                                                        \
-            if (prob->dtype == VLG_F32) return launch_ingest_seg<float, k>(P, W, flip, seg_u8, out_label, out_seg_f32, out_onehot, workspace, st); \
-            return launch_ingest_seg<__nv_bfloat16, k>(P, W, flip, seg_u8, out_label, out_seg_f32, out_onehot, workspace, st);     \
-        }
-        VLG_FOR_EACH_K(X)
-#undef X
-        return fail(VLG_ERR_UNSUPPORTED, "K not compiled in");
+        return with_type_k(prob, [&](auto t, auto k) {
+            return launch_ingest_seg<typename decltype(t)::type, decltype(k)::value>(P, W, flip, seg_u8, out_label, out_seg_f32,
+                                                                                     out_onehot, workspace, st);
+        });
     }
     return rc;
 }
@@ -1298,15 +1248,13 @@ int vlg_ingest(const vlg_problem_t *prob, const uint8_t *frames_u8, const float 
 int vlg_pixel_loss_fwd_bwd(const vlg_problem_t *prob, const void *out_rgb, const void *tgt_rgb, const void *logits,
                            const int64_t *tgt_label, float *loss_out, void *d_out_rgb, void *d_logits,
                            int64_t *out_argmax, void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = check_problem(prob);
-    if (rc) return rc;
-    const WsLayout L = ws_layout(prob, 0);
-    if (!workspace || workspace_bytes < L.total) return fail(VLG_ERR_WORKSPACE, "workspace too small: need %zu bytes", L.total);
+    if (int rc = check_problem(prob)) return rc;
+    WsLayout L;
+    if (int rc = workspace_at(prob, 0, workspace, workspace_bytes, &L)) return rc;
     if ((out_rgb == nullptr) != (tgt_rgb == nullptr)) return fail(VLG_ERR_ARG, "out_rgb and tgt_rgb go together");
     if ((logits == nullptr) != (tgt_label == nullptr)) return fail(VLG_ERR_ARG, "logits and tgt_label go together");
-    rc = run_pass1(prob, false, out_rgb, logits, nullptr, tgt_rgb, tgt_label, nullptr, d_out_rgb, d_logits,
-                   d_out_rgb != nullptr || d_logits != nullptr, out_argmax, loss_out, workspace, L, (cudaStream_t)stream);
-    return rc;
+    return run_pass1(prob, false, out_rgb, logits, nullptr, tgt_rgb, tgt_label, nullptr, d_out_rgb, d_logits,
+                     d_out_rgb != nullptr || d_logits != nullptr, out_argmax, loss_out, L, (cudaStream_t)stream);
 }
 
 int vlg_frame_affine(const vlg_problem_t *prob, const float *in_rgb, int32_t in_is_nchw, const float *a3, const float *b3,
@@ -1325,8 +1273,9 @@ int vlg_frame_affine(const vlg_problem_t *prob, const float *in_rgb, int32_t in_
         FrameAffine fa;
         for (int c = 0; c < 3; ++c) { fa.a[c] = a3[c]; fa.b[c] = b3[c]; }
         fa.denorm = denormalize ? 1 : 0;
-        rc = prob->dtype == VLG_F32 ? launch_frame_affine<float>(prob, fa, in_rgb, in_is_nchw != 0, flip_w ? 1 : 0, out_rgb, st)
-                                    : launch_frame_affine<__nv_bfloat16>(prob, fa, in_rgb, in_is_nchw != 0, flip_w ? 1 : 0, out_rgb, st);
+        rc = with_type(prob->dtype, [&](auto t) {
+            return launch_frame_affine<typename decltype(t)::type>(prob, fa, in_rgb, in_is_nchw != 0, flip_w ? 1 : 0, out_rgb, st);
+        });
         if (rc) return rc;
     }
     if (label_in) {

@@ -119,21 +119,24 @@ __device__ __forceinline__ void reduce_partials_block(const ReduceParams &p, dou
     }
 }
 
-// Layout of the d(loss)/d(warped layout) staging buffer between pass 1 and pass 2: chunk-planar,
-// [n][K/CPC][H*W][CPC] with CPC = 4 channels (one 128-bit word) when K % 4 == 0, else 1.
-template <int K> __host__ __device__ constexpr int dout_cpc() { return K % 4 == 0 ? 4 : 1; }
-template <int K>
-__host__ __device__ __forceinline__ int64_t dout_index(int64_t n, int64_t HW, int64_t px, int k) {
-    constexpr int CPC = dout_cpc<K>();
-    return ((n * (K / CPC) + k / CPC) * HW + px) * CPC + k % CPC;
-}
-
+// The arrays of a workspace (ws_layout); NULL where the problem allocates none.
 struct WsLayout {
-    size_t header, tile_flags, tile_disp, seg_cnt, partials, partials_rgb, partials_lay, flagged, dout_rgb, dout_lay, far_acc, far_list, total;
-    size_t rec_code, rec_frac;   // tap records of pass 1 for pass 2 (pitched rows)
-    int64_t n_blocks;
+    WsHeader *hdr;
+    uint32_t *tile_flags;
+    float *tile_disp;
+    uint32_t *seg_cnt;           // NULL under VLG_FLAG_FAR_WIDE (its space stays reserved)
+    float *partials, *partials_rgb, *partials_lay;
+    int *flagged;
+    // with a source gradient only
+    float *dout_rgb, *dout_lay;
+    uint32_t *rec_code;          // tap records of pass 1 for pass 2 (pitched rows)
+    float2 *rec_frac;
+    long long *far_acc;          // far_acc / far_list: NULL under VLG_FLAG_NO_FAR_PATH
+    int4 *far_list;
     int64_t pitch;               // row pitch (pixels) of dout_rgb / rec_code / rec_frac: W rounded up to 4, so that every
                                  // row starts on a 16-byte boundary and the arrays can be described by TMA tensor maps
+    size_t zero_bytes;           // header .. seg_cnt: what pass 1 resets with one memset
+    size_t total;
 };
 
 // ---------------------------------------------------------------- tiling of pass 1
