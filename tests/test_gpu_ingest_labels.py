@@ -83,20 +83,29 @@ def test_ingest_feeds_the_fused_op():
 
 
 # ------------------------------------------------------------------ label-source fused op
+F32, BF16 = torch.float32, torch.bfloat16
 LAB_CASES = [
-    # N, H, W, K, sigma, far_frac, w_tv, padding, half-pixel flow
-    (2, 128, 256, 20, 4.0, 0.0, 0.5, "border", False),       # BASELINE config 1
-    (2, 61, 93, 20, 3.0, 0.0, 0.3, "zeros", True),           # ragged, zeros padding, exact ties between classes
-    (1, 375, 1242, 20, 48.0, 0.05, 0.1, "border", False),    # KITTI-shaped, large displacement
-    (1, 40, 72, 19, 2.0, 0.0, 1.0, "border", False),         # odd K: nothing in this kernel depends on K % 4
-    (1, 33, 35, 5, 2.0, 0.0, 0.0, "zeros", False),
+    # N, H, W, K, sigma, far_frac, w_tv, padding, half-pixel flow, rgb dtype
+    (2, 128, 256, 20, 4.0, 0.0, 0.5, "border", False, F32),       # BASELINE config 1
+    (2, 61, 93, 20, 3.0, 0.0, 0.3, "zeros", True, F32),           # ragged, zeros padding, exact ties between classes
+    (1, 375, 1242, 20, 48.0, 0.05, 0.1, "border", False, F32),    # KITTI-shaped, large displacement
+    (1, 40, 72, 19, 2.0, 0.0, 1.0, "border", False, F32),         # odd K: nothing in this kernel depends on K % 4
+    (1, 33, 35, 5, 2.0, 0.0, 0.0, "zeros", False, F32),
+    # bf16 rgb (rgb_strip_kernel<bf16>); the dense comparison then takes lay_tile_kernel (even W) / pass1_kernel (odd W)
+    (2, 128, 256, 20, 4.0, 0.0, 0.5, "border", False, BF16),
+    (2, 61, 93, 20, 3.0, 0.0, 0.3, "zeros", True, BF16),
+    (1, 375, 1242, 20, 48.0, 0.05, 0.1, "border", False, BF16),
+    (1, 33, 35, 5, 2.0, 0.0, 0.0, "zeros", False, BF16),
 ]
 
 
-@pytest.mark.parametrize("case", LAB_CASES, ids=[f"{c[0]}x{c[1]}x{c[2]}k{c[3]}s{c[4]}{c[7]}" for c in LAB_CASES])
+@pytest.mark.parametrize("case", LAB_CASES, ids=[f"{c[0]}x{c[1]}x{c[2]}k{c[3]}s{c[4]}{c[7]}" + ("" if c[9] == F32 else "-bf16")
+                                                 for c in LAB_CASES])
 def test_label_source_op_vs_oracle_and_dense_path(case):
-    N, H, W, K, sigma, far, w_tv, padding, half = case
+    N, H, W, K, sigma, far, w_tv, padding, half, dt = case
     d = _make_case(N, H, W, K, sigma, seed=1024, layout="onehot", far_frac=far)
+    # bf16 rgb: the oracle sees the same bf16-rounded values, in fp32; the one-hot layout is exact in bf16
+    d = dict(d, **{k: d[k].to(dt).float() for k in ("src_rgb", "src_layout", "tgt_rgb")})
     flow = torch.round(d["flow"] * 2) / 2 if half else d["flow"]
     lab_src = d["src_layout"].argmax(1)
     ref = TO.warp_loss_fwd_bwd(d["src_rgb"], d["src_layout"], flow, d["tgt_rgb"], d["tgt_label"], w_tv=w_tv, padding_mode=padding)
@@ -104,7 +113,8 @@ def test_label_source_op_vs_oracle_and_dense_path(case):
                                  dtype=torch.float64)
     cfg = vlg_b200.WarpLossConfig(w_tv=w_tv, padding_mode=padding, want_argmax=True)
     f = flow.to(DEV).requires_grad_(True)
-    total, vec, arg = vlg_b200.warp_loss_labels(_cl(d["src_rgb"]), lab_src.to(DEV), f, _cl(d["tgt_rgb"]), d["tgt_label"].to(DEV), cfg, n_classes=K)
+    total, vec, arg = vlg_b200.warp_loss_labels(_cl(d["src_rgb"].to(dt)), lab_src.to(DEV), f, _cl(d["tgt_rgb"].to(dt)), d["tgt_label"].to(DEV), cfg,
+                                                n_classes=K)
     total.backward()
     assert torch.equal(arg.cpu(), ref["argmax"])                                  # bit-exact layouts
     want = np.array([ref["terms"][k].item() for k in TERMS])
@@ -115,15 +125,16 @@ def test_label_source_op_vs_oracle_and_dense_path(case):
     # against the dense path of the product on the one-hot layout: same argmax, loss vector and d_flow to fp32 rounding
     if K % 4 == 0:
         f2 = flow.to(DEV).requires_grad_(True)
-        t2, v2, a2 = vlg_b200.warp_loss(_cl(d["src_rgb"]), _cl(d["src_layout"]), f2, _cl(d["tgt_rgb"]), d["tgt_label"].to(DEV), cfg)
+        t2, v2, a2 = vlg_b200.warp_loss(_cl(d["src_rgb"].to(dt)), _cl(d["src_layout"].to(dt)), f2, _cl(d["tgt_rgb"].to(dt)),
+                                        d["tgt_label"].to(DEV), cfg)
         t2.backward()
         assert torch.equal(a2, arg)
         np.testing.assert_allclose(vec.cpu().numpy()[:6], v2.cpu().numpy()[:6], rtol=5e-6, atol=1e-7)
         assert_grad_parity(f.grad, f2.grad, None, 5e-6, "d_flow label source vs dense source")
     # validation mode (no gradient) and two runs bitwise identical
     with torch.no_grad():
-        t3, v3, a3 = vlg_b200.warp_loss_labels(_cl(d["src_rgb"]), lab_src.to(DEV), flow.to(DEV), _cl(d["tgt_rgb"]), d["tgt_label"].to(DEV), cfg,
-                                               n_classes=K)
+        t3, v3, a3 = vlg_b200.warp_loss_labels(_cl(d["src_rgb"].to(dt)), lab_src.to(DEV), flow.to(DEV), _cl(d["tgt_rgb"].to(dt)),
+                                               d["tgt_label"].to(DEV), cfg, n_classes=K)
     assert torch.equal(v3[:6], vec[:6]) and torch.equal(a3, arg)
 
 
